@@ -2,6 +2,7 @@
 """bench.py -- tasks/sec of one meta-batch forward + loss + backward (the BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--precision P]
+                    [--dump-outputs DIR]
 
 Default workload = BASELINE.json configs[1]: ConvCNP(1,1) default constructor (I=384 induced points, 3 ResConvBlocks
 k=11), meta-batch 256 tasks PER GPU, 128 context / 128 target points, fp32 storage, synthetic data (random-init
@@ -11,6 +12,11 @@ flat gradient is all-reduced (NCCL) inside the timed region.  One JSON line on s
 `--impl reference` times the reference's own CPU path (the unmodified upstream package installed under baseline/_ref by
 baseline/install_ref.sh; the oracle port only if that directory did not travel) on a bounded sample of the same workload.
 The default run also carries short runs of the other BASELINE configs as `other_workloads`.
+
+`--dump-outputs DIR` writes what the last timed step of the workload returned to its caller (rank 0): the loss as
+DIR/loss.npy and every parameter's gradient as DIR/grad.<parameter name>.npy, float32, at most 64 MB in all (beyond that
+the largest arrays are replaced by a fixed, seeded sample of their entries: see dump_outputs).  Weights and inputs are
+seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -221,9 +227,10 @@ def _reference_model(fam):
     return m.train(), npf
 
 
-def cpu_reference_timing(wl, steps, warmup, budget_s=25.0):
+def cpu_reference_timing(wl, steps, warmup, budget_s=None):
     """The reference's CPU path on the host cores: fwd + loss + bwd of a bounded sample of the workload (Bc tasks per step,
-    same C / T / image size as the GPU workload).  kind="reference": the unmodified upstream package (baseline/_ref, through
+    same C / T / image size as the GPU workload).  Times exactly `steps` steps, or with `budget_s` as many as fit in that many
+    seconds (at least one, at most `steps`).  kind="reference": the unmodified upstream package (baseline/_ref, through
     its own public API: npf.<Model>(...)(X_cntxt, Y_cntxt, X_trgt, Y_trgt) -> npf.<Loss> -> backward); kind="port": the
     oracle's torch-CPU restatement, only when baseline/_ref did not travel."""
     avail = len(os.sched_getaffinity(0)) if hasattr(os, "sched_getaffinity") else (os.cpu_count() or 1)
@@ -282,7 +289,7 @@ def cpu_reference_timing(wl, steps, warmup, budget_s=25.0):
     w = max(1, min(warmup, int(3.0 / max(one, 1e-3))))
     for _ in range(w - 1):
         step()
-    k = max(1, min(steps, int(budget_s / max(one, 1e-3))))
+    k = steps if budget_s is None else max(1, min(steps, int(budget_s / max(one, 1e-3))))
     t0 = time.perf_counter()
     for _ in range(k):
         step()
@@ -298,9 +305,10 @@ def make_loss(name, reduction="mean"):
     return dict(cnpf=npf_b200.CNPFLoss, nll=npf_b200.NLLLossLNPF, elbo=npf_b200.ELBOLossLNPF)[name](reduction=reduction)
 
 
-def run_ours(wl_name, args, ctx, steps, warmup, full):
+def run_ours(wl_name, args, ctx, steps, warmup, full, capture_outputs=False):
     """One workload through the public API (GraphedStep): device-timed region with resident inputs, the end-to-end region
-    from pinned host buffers, and the per-kernel breakdown.  `full` adds the fp32-path timing."""
+    from pinned host buffers, and the per-kernel breakdown.  `full` adds the fp32-path timing; `capture_outputs` returns the
+    loss and the gradients of the last timed step as numpy arrays."""
     import npf_b200
     from npf_b200 import _cabi, ops
     from npf_b200.parallel import FlatGradients
@@ -350,18 +358,25 @@ def run_ours(wl_name, args, ctx, steps, warmup, full):
     n0 = ops.launch_count()
     barrier()
     t_wall = time.perf_counter()
+    timed = 0                               # steps the loop ran: what the rates below and the JSON line's `steps` count
     for i in range(steps):
         flush.fill_(float(i))
         evs[i][0].record()
-        step(dev_inputs[i % n_sets])
+        loss = step(dev_inputs[i % n_sets])
         evs[i][1].record()
+        timed += 1
         if rank == 0 and i % 8 == 4:
             sampler.sample_now()            # under load: the GPU is several replays behind the host here
     barrier()
     t_wall = time.perf_counter() - t_wall
-    launches = ops.launch_count() - n0 if gstep is None else gstep.last_launches * steps   # replays launch the recorded kernels
-    dev_ms = sum(a.elapsed_time(b) for a, b in evs)
+    launches = ops.launch_count() - n0 if gstep is None else gstep.last_launches * timed   # replays launch the recorded kernels
+    dev_ms = sum(a.elapsed_time(b) for a, b in evs[:timed])
     clocks = sampler.stop() if rank == 0 else None
+    outputs = None
+    if capture_outputs:
+        # what the caller of the last timed step received, copied before the regions below overwrite the loss and the gradients
+        outputs = {"loss": loss.detach().float().cpu().numpy()}
+        outputs.update({f"grad.{n}": p.grad.detach().float().cpu().numpy() for n, p in model.named_parameters() if p.grad is not None})
 
     # ---- timed region 2: end to end through the public API from pinned host buffers --------------------------------
     # Public API for host-resident batches: npf_b200.PipelinedStep(GraphedStep) -- every step copies its own inputs host -> device
@@ -432,11 +447,37 @@ def run_ours(wl_name, args, ctx, steps, warmup, full):
     flat.detach()
     del gstep, model, flat, dev_inputs, host_inputs
     torch.cuda.empty_cache()
-    tasks = B * world * steps
-    return dict(wl=wl, B=B, steps=steps, warmup=warm, value=tasks / (dev_ms * 1e-3), ms_per_step=dev_ms / steps,
-                e2e=dict(value=tasks / (e2e_ms * 1e-3), unit="tasks/s", h2d_bytes_per_step=h2d, d2h_bytes_per_step=4),
-                launches=launches, wall_ms_per_step=t_wall * 1e3 / steps, clocks=clocks, ktimes=ktimes, shaped=shaped, n_prof=n_prof,
-                fp32_path=fp32_path)
+    tasks = B * world * timed
+    return dict(wl=wl, B=B, steps=timed, warmup=warm, value=tasks / (dev_ms * 1e-3), ms_per_step=dev_ms / timed,
+                e2e=dict(value=B * world * steps / (e2e_ms * 1e-3), unit="tasks/s", h2d_bytes_per_step=h2d, d2h_bytes_per_step=4),
+                launches=launches, wall_ms_per_step=t_wall * 1e3 / timed, clocks=clocks, ktimes=ktimes, shaped=shaped, n_prof=n_prof,
+                fp32_path=fp32_path, outputs=outputs)
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, outputs, limit_bytes=DUMP_LIMIT_BYTES):
+    """Writes every array as out_dir/<name>.npy in float32, at most `limit_bytes` in all.  When the arrays hold more, the
+    largest ones are cut to a common number of entries: a sample drawn at seeded positions (the same on every run) from the
+    flattened array, kept in index order, so two runs still compare entry for entry; smaller arrays stay whole."""
+    import numpy as np
+    arrays = {name: np.asarray(a, dtype=np.float32) for name, a in outputs.items()}
+    budget = (limit_bytes - 128 * len(arrays)) // 4          # float32 entries, after one 128-byte .npy header per file
+    cap = None
+    if sum(a.size for a in arrays.values()) > budget:
+        sizes = sorted(a.size for a in arrays.values())
+        for i, n in enumerate(sizes):
+            share = budget // (len(sizes) - i)
+            if n > share:
+                cap = share
+                break
+            budget -= n
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        if cap is not None and a.size > cap:
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, cap, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def workload_config(name, world, no_graph):
@@ -451,7 +492,7 @@ def workload_config(name, world, no_graph):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=100)
+    ap.add_argument("--steps", type=int, default=100, help="number of timed steps")
     ap.add_argument("--warmup", type=int, default=10)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="convcnp1d_b256_c128_t128", choices=list(WORKLOADS))
@@ -462,7 +503,12 @@ def main():
     ap.add_argument("--no-others", action="store_true", help="skip the short runs of the other BASELINE workloads (`other_workloads`)")
     ap.add_argument("--no-graph", action="store_true", help="eager launches instead of the CUDA-graph replay of the step (npf_b200.GraphedStep)")
     ap.add_argument("--kernel-times", action="store_true", help="print the per-kernel CUDA-event breakdown to stderr")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the loss and the gradients of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     wl = WORKLOADS[args.workload]
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -496,7 +542,9 @@ def main():
                flush=torch.empty(256 * 1024 * 1024 // 4, device=dev))
     peaks = measured_peaks()
 
-    r = run_ours(args.workload, args, ctx, args.steps, args.warmup, full=True)
+    r = run_ours(args.workload, args, ctx, args.steps, args.warmup, full=True, capture_outputs=bool(args.dump_outputs))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, r["outputs"])
     # short runs of the other BASELINE workloads, so that one driver-run line shows every config (same protocol, fewer steps)
     others = {}
     if not args.no_others and args.workload == "convcnp1d_b256_c128_t128":
@@ -515,7 +563,7 @@ def main():
 
     ktimes, n_prof = r["ktimes"], r["n_prof"]
     roof, roof_table = roofline(wl, ktimes, n_prof, r["B"], peaks, r["shaped"])
-    line = dict(metric="tasks/sec (meta-batch fwd+bwd)", value=r["value"], unit="tasks/s", n_gpus=world, steps=args.steps,
+    line = dict(metric="tasks/sec (meta-batch fwd+bwd)", value=r["value"], unit="tasks/s", n_gpus=world, steps=r["steps"],
                 warmup=r["warmup"], ms_per_step=r["ms_per_step"], higher_is_better=True, scaling="weak",
                 vs_baseline=None, dtype={"fp32": "f32", "bf16": "bf16", "bf16x3": "bf16x3 (fp32-equivalent)"}[args.precision],
                 data="synthetic", config=workload_config(args.workload, world, args.no_graph), clocks=r["clocks"],
