@@ -15,8 +15,6 @@
 //   Q, K   K-major over d :  (d/8)*LBO + (row/8)*128 + (row%8)*16 + (d%8)*2,   LBO = rows*16
 //   P      K-major over key: (key/8)*2048 + (q/8)*128 + (q%8)*16 + (key%8)*2
 //   V      MN-major (N = channel c, K = key): (key/8)*LBO + (c/8)*128 + (key%8)*16 + (c%8)*2,  LBO = (Dv/8)*128
-#include <cstdlib>
-
 #include "tc_common.cuh"
 
 namespace npf {
@@ -75,22 +73,8 @@ __device__ __forceinline__ void stage_rows_kmajor(uint8_t* hi, uint8_t* lo, cons
 // attention has |logit| ~ 1e2): with NSPLIT == 3 the product Q K^T uses three bf16 terms per operand and the six
 // cross products down to 2^-24: hh, hm, mh, mm, hl, lh.
 template <int NSPLIT>
-__device__ __forceinline__ void mma_logits(uint32_t d, uint32_t a_h, uint32_t a_m, uint32_t a_l, uint32_t b_h, uint32_t b_m, uint32_t b_l,
-                                           uint32_t lbo, uint32_t idesc, uint32_t acc) {
-    umma_bf16(d, make_desc(a_h, lbo, 128), make_desc(b_h, lbo, 128), idesc, acc);
-    if (NSPLIT == 3) {
-        umma_bf16(d, make_desc(a_h, lbo, 128), make_desc(b_m, lbo, 128), idesc, 1);
-        umma_bf16(d, make_desc(a_m, lbo, 128), make_desc(b_h, lbo, 128), idesc, 1);
-        umma_bf16(d, make_desc(a_m, lbo, 128), make_desc(b_m, lbo, 128), idesc, 1);
-        umma_bf16(d, make_desc(a_h, lbo, 128), make_desc(b_l, lbo, 128), idesc, 1);
-        umma_bf16(d, make_desc(a_l, lbo, 128), make_desc(b_h, lbo, 128), idesc, 1);
-    }
-}
-
-// the same product with different leading-dimension offsets for the two operands (tiles with different row counts)
-template <int NSPLIT>
-__device__ __forceinline__ void mma_logits2(uint32_t d, uint32_t a_h, uint32_t a_m, uint32_t a_l, uint32_t a_lbo, uint32_t b_h, uint32_t b_m, uint32_t b_l,
-                                            uint32_t b_lbo, uint32_t idesc, uint32_t acc) {
+__device__ __forceinline__ void mma_logits(uint32_t d, uint32_t a_h, uint32_t a_m, uint32_t a_l, uint32_t a_lbo, uint32_t b_h, uint32_t b_m, uint32_t b_l,
+                                           uint32_t b_lbo, uint32_t idesc, uint32_t acc) {
     umma_bf16(d, make_desc(a_h, a_lbo, 128), make_desc(b_h, b_lbo, 128), idesc, acc);
     if (NSPLIT == 3) {
         umma_bf16(d, make_desc(a_h, a_lbo, 128), make_desc(b_m, b_lbo, 128), idesc, 1);
@@ -189,8 +173,8 @@ __global__ void __launch_bounds__(128) xattn_fwd_tc_kernel(AttnTcParams p) {
             tc_fence_after();
             for (int ks = 0; ks < D / 16; ++ks) {
                 const uint32_t oq = (uint32_t)ks * 2u * q_lbo, ok = (uint32_t)ks * 2u * k_lbo;
-                mma_logits2<NSPLIT>(tmem, smem_u32(q_hi) + oq, smem_u32(q_lo) + oq, smem_u32(q_l2) + oq, q_lbo, smem_u32(k_hi) + ok, smem_u32(k_lo) + ok,
-                                    smem_u32(k_l2) + ok, k_lbo, idesc_s, ks > 0);
+                mma_logits<NSPLIT>(tmem, smem_u32(q_hi) + oq, smem_u32(q_lo) + oq, smem_u32(q_l2) + oq, q_lbo, smem_u32(k_hi) + ok, smem_u32(k_lo) + ok,
+                                   smem_u32(k_l2) + ok, k_lbo, idesc_s, ks > 0);
             }
             umma_commit(&bar_s);
         }
@@ -299,24 +283,26 @@ static int launch_fwd_kc(AttnTcParams& p, int B, cudaStream_t st) {
 }
 template <int NSPLIT, int DV>
 static int launch_fwd(AttnTcParams& p, int B, cudaStream_t st) {
-    static const int kc = [] { const char* e = getenv("NPF_XATTN_KC"); return e && atoi(e) == 128 ? 128 : (e && atoi(e) == 64 ? 64 : 0); }();
     // 64-key chunks when there are enough CTAs to fill four per SM and more than one chunk of keys anyway
     const long ctas = (long)cdiv(p.Tq, kQB) * p.H * B;
-    const bool small = kc == 64 || (kc == 0 && p.Tk > 64 && ctas >= 2L * kNumSMs);
+    const bool small = p.Tk > 64 && ctas >= 2L * kNumSMs;
     return small ? launch_fwd_kc<NSPLIT, DV, 64>(p, B, st) : launch_fwd_kc<NSPLIT, DV, 128>(p, B, st);
 }
 
 // ----------------------------------------------------------------------------------------------------------------
-// Backward.  One CTA per (task, head, 128-key block); loops over the 128-query blocks.  256 threads: thread t owns
-// TMEM lane / query row r = t & 127 and the key-column half t >> 7 of the 128 x 128 score tile.
-//   S = Q K^T, dP = dO V^T                 (two MMAs, M=128 N=128 K=D|Dv)                      TMEM [0,128), [128,256)
-//   P = exp(S*scale - lse), dS = P (dP - Di) scale   -> bf16 hi/lo into the shared operand tiles Pt / dSt
-//   dV += P^T dO,  dK += dS^T Q            (M = keys, K = queries; accumulate over query blocks) TMEM [320,..), [288,..)
-//   dQ_blk = dS K                          (M = queries, K = keys)                               TMEM [256,..) -> atomics
-// Every staged tile uses ONE physical layout: 16-byte rows of 8 consecutive columns, 8 rows = a 128-byte core matrix,
-// row groups 128 B apart, column chunks 2048 B apart.  Read with (LBO=2048, SBO=128) it is a K-major operand over its
-// columns; read with (LBO=128, SBO=2048) and the MN-major flag it is the TRANSPOSED operand -- so Q, dO, K, P and dS
-// are staged once and serve both of their roles.
+// Backward.  One CTA per (task, head, 128-key block); loops over 64-query blocks with the score tile TRANSPOSED (TMEM
+// lane = key), so that two CTAs fit an SM: a CTA's phases (stage -> MMA -> exp -> MMA -> atomics) are strictly serial, and
+// the other CTA's work fills its hand-offs.  Per 64-query block:
+//   S^T = K Q^T, dP^T = V dO^T                 (M = 128 keys, N = 64 queries, K = D | Dv: every operand in its natural row-major staging)
+//   thread (key r, query half) : P^T = exp2(S^T scale - lse[q]), dS^T = P^T (dP^T - Di[q]) scale      -> [128 keys x 64 q] bf16 hi / lo images
+//   dV += P^T dO,  dK += dS^T Q                (A = the images as stored, K-major over q; B = dO / Q read through the transposed view)
+//   dQ_blk = dS K                               (A = transposed view of the dS^T image: its M extent is the 64 queries; the MMA runs with
+//                                                M = 128 and the upper 64 accumulator rows, fed by whatever follows the image, are never read)
+// 94 KB of shared memory (head dim 16) and 224 TMEM columns per CTA.
+// Every staged tile uses ONE physical layout: 16-byte rows of 8 consecutive columns, 8 rows = a 128-byte core matrix, row
+// groups 128 B apart, column chunks rows x 16 B apart (CHK = 2048 B in the 128-row tiles, CHQ = 1024 B in the 64-row ones).
+// Read with (LBO = chunk stride, SBO = 128) it is a K-major operand over its columns; read with (LBO = 128, SBO = chunk
+// stride) and the MN-major flag it is the TRANSPOSED operand -- so Q, dO, K, P and dS are staged once and serve both roles.
 // ----------------------------------------------------------------------------------------------------------------
 template <int NSPLIT>
 __device__ __forceinline__ void mma3(uint32_t d, uint32_t a_hi, uint32_t a_lo, uint32_t a_lbo, uint32_t a_sbo, uint32_t b_hi, uint32_t b_lo,
@@ -328,194 +314,6 @@ __device__ __forceinline__ void mma3(uint32_t d, uint32_t a_hi, uint32_t a_lo, u
     }
 }
 
-template <int NSPLIT>
-__global__ void __launch_bounds__(256, 1) xattn_bwd_tc_kernel(AttnTcParams p) {
-    extern __shared__ __align__(1024) uint8_t smem_raw[];
-    __shared__ __align__(8) uint64_t bar1, bar2;
-    __shared__ uint32_t tmem_slot;
-    __shared__ float s_lse2[128], s_di[128];
-    const int D = p.D, DV = p.Dv;
-    constexpr uint32_t CH = 2048u;                               // column-chunk stride of every tile (128 rows x 16 B)
-    const uint32_t t_small = (uint32_t)(D >> 3) * CH, t_small_v = (uint32_t)(DV >> 3) * CH, t_big = 16u * CH;
-    uint8_t* kt = smem_raw;
-    uint8_t* vt = kt + t_small;
-    uint8_t* qt = vt + t_small_v;
-    uint8_t* dot_ = qt + t_small;
-    uint8_t* pt = dot_ + t_small_v;
-    uint8_t* dst = pt + t_big;
-    const uint32_t half = 2u * t_small + 2u * t_small_v + 2u * t_big;
-    const uint32_t LO = half;                                     // byte offset of the "lo" copies (NSPLIT == 3)
-    uint8_t* kt_l2 = smem_raw + 2 * half; uint8_t* qt_l2 = kt_l2 + t_small;   // third bf16 term of K and Q (logits only)
-
-    const int tid = threadIdx.x, warp = tid >> 5;
-    const int r = tid & 127, chalf = tid >> 7;
-    const int kb = blockIdx.x, h = blockIdx.y, b = blockIdx.z;
-    const long ldq = (long)p.H * D, ldv = (long)p.H * DV;
-    const float* Qb = p.Q + ((long)b * p.Tq) * ldq + h * D;
-    const float* Kb = p.K + ((long)b * p.Tk) * ldq + h * D;
-    const float* Vb = p.V + ((long)b * p.Tk) * ldv + h * DV;
-    const float* Ob = p.O + ((long)b * p.Tq) * ldv + h * DV;
-    const float* Gb = p.dO + ((long)b * p.Tq) * ldv + h * DV;
-
-    if (warp == 0) tmem_alloc(&tmem_slot, 512);
-    if (tid == 0) { mbar_init(&bar1, 1); mbar_init(&bar2, 1); }
-    const int key0 = kb * 128;
-    if (tid < 128) {
-        const bool k_ok = key0 + tid < p.Tk;
-        stage_rows_kmajor<NSPLIT>(kt, kt + LO, Kb + (long)key0 * ldq, ldq, tid, k_ok, D, 128, NSPLIT == 3 ? kt_l2 : nullptr);
-        stage_rows_kmajor<NSPLIT>(vt, vt + LO, Vb + (long)key0 * ldv, ldv, tid, k_ok, DV, 128);
-    }
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem = tmem_slot;
-    const uint32_t lane_addr = (uint32_t)(32 * (warp & 3)) << 16;
-    const uint32_t T_S = 0, T_DP = 128, T_DQ = 256, T_DK = 288, T_DV = 320;
-    const uint32_t idesc_sp = make_idesc(128, 128, 0, 0);
-    const uint32_t idesc_dv = make_idesc(128, DV, 1, 1), idesc_dk = make_idesc(128, D, 1, 1), idesc_dq = make_idesc(128, D, 0, 1);
-    const float sl2 = p.scale * 1.4426950408889634f;
-    const uint32_t s_kt = smem_u32(kt), s_vt = smem_u32(vt), s_qt = smem_u32(qt), s_dot = smem_u32(dot_), s_pt = smem_u32(pt), s_dst = smem_u32(dst);
-
-    uint32_t ph = 0, acc_kv = 0;
-    for (int q0 = 0; q0 < p.Tq; q0 += 128) {
-        if (tid < 128) {   // stage this query block: Q, dO tiles + per-row lse and Di = dO . O
-            const int q = q0 + tid;
-            const bool q_ok = q < p.Tq;
-            stage_rows_kmajor<NSPLIT>(qt, qt + LO, Qb + (long)q0 * ldq, ldq, tid, q_ok, D, 128, NSPLIT == 3 ? qt_l2 : nullptr);
-            stage_rows_kmajor<NSPLIT>(dot_, dot_ + LO, Gb + (long)q0 * ldv, ldv, tid, q_ok, DV, 128);
-            float di = 0.f;
-            if (q_ok)
-                for (int c = 0; c < DV; ++c) di = fmaf(__ldg(Gb + (long)q * ldv + c), __ldg(Ob + (long)q * ldv + c), di);
-            s_di[tid] = di;
-            s_lse2[tid] = q_ok ? __ldg(p.LSE + ((long)b * p.H + h) * p.Tq + q) * 1.4426950408889634f : INFINITY;   // +inf -> P = 0
-        }
-        fence_async_smem();
-        tc_fence_before();
-        __syncthreads();
-        if (tid == 0) {
-            tc_fence_after();
-            for (int ks = 0; ks < D / 16; ++ks)      // S = Q K^T : both K-major over d, fp32-level product
-                mma_logits<NSPLIT>(tmem + T_S, s_qt + ks * 2 * CH, s_qt + LO + ks * 2 * CH, smem_u32(qt_l2) + ks * 2 * CH, s_kt + ks * 2 * CH,
-                                   s_kt + LO + ks * 2 * CH, smem_u32(kt_l2) + ks * 2 * CH, CH, idesc_sp, ks > 0);
-            for (int ks = 0; ks < DV / 16; ++ks)     // dP = dO V^T
-                mma3<NSPLIT>(tmem + T_DP, s_dot + ks * 2 * CH, s_dot + LO + ks * 2 * CH, CH, 128, s_vt + ks * 2 * CH, s_vt + LO + ks * 2 * CH, CH, 128,
-                             idesc_sp, ks > 0);
-            umma_commit(&bar1);
-        }
-        mbar_wait(&bar1, ph);
-        tc_fence_after();
-
-        {   // P and dS for row r, key columns [64*chalf, 64*chalf + 64)
-            const float lse2 = s_lse2[r], di = s_di[r];
-#pragma unroll 1
-            for (int c0 = 64 * chalf; c0 < 64 * chalf + 64; c0 += 32) {
-                float sv[32], dv[32];
-                tmem_ld32(tmem + lane_addr + T_S + (uint32_t)c0, sv);
-                tmem_ld32(tmem + lane_addr + T_DP + (uint32_t)c0, dv);
-#pragma unroll
-                for (int j = 0; j < 32; ++j) {
-                    const bool ok = key0 + c0 + j < p.Tk;
-                    const float pj = ok ? exp2f(fmaf(sv[j], sl2, -lse2)) : 0.f;
-                    sv[j] = pj;
-                    dv[j] = pj * (dv[j] - di) * p.scale;
-                }
-#pragma unroll
-                for (int g = 0; g < 4; ++g) {
-                    float a8[8], b8[8];
-#pragma unroll
-                    for (int i = 0; i < 8; ++i) { a8[i] = sv[g * 8 + i]; b8[i] = dv[g * 8 + i]; }
-                    const uint32_t off = (uint32_t)((c0 >> 3) + g) * CH + (uint32_t)(r >> 3) * 128u + (uint32_t)(r & 7) * 16u;
-                    *reinterpret_cast<uint4*>(pt + off) = pack8(a8);
-                    *reinterpret_cast<uint4*>(dst + off) = pack8(b8);
-                    if (NSPLIT == 3) {
-                        float l8[8];
-                        split8(a8, l8);
-                        *reinterpret_cast<uint4*>(pt + LO + off) = pack8(l8);
-                        split8(b8, l8);
-                        *reinterpret_cast<uint4*>(dst + LO + off) = pack8(l8);
-                    }
-                }
-            }
-        }
-        fence_async_smem();
-        tc_fence_before();
-        __syncthreads();
-        if (tid == 0) {
-            tc_fence_after();
-            for (int ks = 0; ks < 8; ++ks) {        // reduction over the 128 query rows, 16 per step
-                // dV += P^T dO : A = P read transposed (MN-major: LBO = 128 between 8-row groups, SBO = CH between key chunks)
-                mma3<NSPLIT>(tmem + T_DV, s_pt + ks * 256, s_pt + LO + ks * 256, 128, CH, s_dot + ks * 256, s_dot + LO + ks * 256, 128, CH, idesc_dv,
-                             acc_kv | (uint32_t)(ks > 0));
-                // dK += dS^T Q
-                mma3<NSPLIT>(tmem + T_DK, s_dst + ks * 256, s_dst + LO + ks * 256, 128, CH, s_qt + ks * 256, s_qt + LO + ks * 256, 128, CH, idesc_dk,
-                             acc_kv | (uint32_t)(ks > 0));
-            }
-            for (int ks = 0; ks < 8; ++ks)          // dQ_blk = dS K : reduction over the 128 keys
-                mma3<NSPLIT>(tmem + T_DQ, s_dst + ks * 2 * CH, s_dst + LO + ks * 2 * CH, CH, 128, s_kt + ks * 256, s_kt + LO + ks * 256, 128, CH, idesc_dq,
-                             ks > 0);
-            umma_commit(&bar2);
-        }
-        acc_kv = 1;
-        mbar_wait(&bar2, ph);
-        ph ^= 1;
-        tc_fence_after();
-        if (chalf == 0) {
-            const int q = q0 + r;
-            for (int c0 = 0; c0 < D; c0 += 16) {
-                float v[16];
-                tmem_ld16(tmem + lane_addr + T_DQ + (uint32_t)c0, v);
-                if (q < p.Tq) {
-                    float* d = p.dQ + ((long)b * p.Tq + q) * ldq + h * D + c0;
-#pragma unroll
-                    for (int j = 0; j < 16; j += 4) atomicAdd(reinterpret_cast<float4*>(d + j), make_float4(v[j], v[j + 1], v[j + 2], v[j + 3]));
-                }
-            }
-        }
-        tc_fence_before();
-        __syncthreads();
-    }
-    if (acc_kv) {
-        tc_fence_after();
-        if (chalf == 0) {
-            const int key = key0 + r;
-            for (int c0 = 0; c0 < D; c0 += 16) {
-                float v[16];
-                tmem_ld16(tmem + lane_addr + T_DK + (uint32_t)c0, v);
-                if (key < p.Tk) {
-                    float* d = p.dK + ((long)b * p.Tk + key) * ldq + h * D + c0;
-#pragma unroll
-                    for (int j = 0; j < 16; j += 4) *reinterpret_cast<float4*>(d + j) = make_float4(v[j], v[j + 1], v[j + 2], v[j + 3]);
-                }
-            }
-        } else {
-            const int key = key0 + r;
-            for (int c0 = 0; c0 < DV; c0 += 16) {
-                float v[16];
-                tmem_ld16(tmem + lane_addr + T_DV + (uint32_t)c0, v);
-                if (key < p.Tk) {
-                    float* d = p.dV + ((long)b * p.Tk + key) * ldv + h * DV + c0;
-#pragma unroll
-                    for (int j = 0; j < 16; j += 4) *reinterpret_cast<float4*>(d + j) = make_float4(v[j], v[j + 1], v[j + 2], v[j + 3]);
-                }
-            }
-        }
-        tc_fence_before();
-    }
-    __syncthreads();
-    if (warp == 0) tmem_dealloc(tmem, 512);
-}
-
-// ----------------------------------------------------------------------------------------------------------------
-// Backward, second arrangement: 64-query blocks and the score tile TRANSPOSED (TMEM lane = key), so that two CTAs fit an SM.
-// The kernel above holds P and dS for 128 x 128 scores as bf16 hi / lo images (128 KB) and 352 TMEM columns: one CTA per SM, and
-// its phases (stage -> MMA -> exp -> MMA -> atomics) are strictly serial, so the SM idles through every hand-off.  Here, per 64-query block:
-//   S^T = K Q^T, dP^T = V dO^T                 (M = 128 keys, N = 64 queries, K = D | Dv: every operand in its natural row-major staging)
-//   thread (key r, query half) : P^T = exp2(S^T scale - lse[q]), dS^T = P^T (dP^T - Di[q]) scale      -> [128 keys x 64 q] bf16 hi / lo images
-//   dV += P^T dO,  dK += dS^T Q                (A = the images as stored, K-major over q; B = dO / Q read through the transposed view)
-//   dQ_blk = dS K                               (A = transposed view of the dS^T image: its M extent is the 64 queries; the MMA runs with
-//                                                M = 128 and the upper 64 accumulator rows, fed by whatever follows the image, are never read)
-// 94 KB of shared memory (head dim 16) and 224 TMEM columns per CTA.
-// ----------------------------------------------------------------------------------------------------------------
 template <int NSPLIT>
 __global__ void __launch_bounds__(256, 2) xattn_bwd_tc_q64_kernel(AttnTcParams p) {
     extern __shared__ __align__(1024) uint8_t smem_raw[];
@@ -588,8 +386,8 @@ __global__ void __launch_bounds__(256, 2) xattn_bwd_tc_q64_kernel(AttnTcParams p
         if (tid == 0) {
             tc_fence_after();
             for (int ks = 0; ks < D / 16; ++ks)      // S^T = K Q^T : both K-major over d, fp32-level product
-                mma_logits2<NSPLIT>(tmem + T_S, s_kt + ks * 2 * CHK, s_kt + LO + ks * 2 * CHK, smem_u32(kt_l2) + ks * 2 * CHK, CHK, s_qt + ks * 2 * CHQ,
-                                    s_qt + LO + ks * 2 * CHQ, smem_u32(qt_l2) + ks * 2 * CHQ, CHQ, idesc_sp, ks > 0);
+                mma_logits<NSPLIT>(tmem + T_S, s_kt + ks * 2 * CHK, s_kt + LO + ks * 2 * CHK, smem_u32(kt_l2) + ks * 2 * CHK, CHK, s_qt + ks * 2 * CHQ,
+                                   s_qt + LO + ks * 2 * CHQ, smem_u32(qt_l2) + ks * 2 * CHQ, CHQ, idesc_sp, ks > 0);
             for (int ks = 0; ks < DV / 16; ++ks)     // dP^T = V dO^T
                 mma3<NSPLIT>(tmem + T_DP, s_vt + ks * 2 * CHK, s_vt + LO + ks * 2 * CHK, CHK, 128, s_dot + ks * 2 * CHQ, s_dot + LO + ks * 2 * CHQ, CHQ, 128,
                              idesc_sp, ks > 0);
@@ -714,46 +512,24 @@ int xattn_bwd_tc(const float* Q, const float* K, const float* V, const float* O,
     auto al = [](const void* q) { return (reinterpret_cast<uintptr_t>(q) & 15) == 0; };
     if (!attn_tc_ok(p) || !al(O) || !al(dO) || !al(dQ) || !al(dK) || !al(dV) || Tq < 1) return NPF_ENOTSUP;
     const bool x3 = precision == NPF_PREC_BF16X3;
-    {   // 64-query arrangement (two CTAs per SM) unless switched off
-        static const bool q64 = [] { const char* e = getenv("NPF_XATTN_BWD_Q64"); return !(e && e[0] == '0'); }();
-        const size_t half64 = (size_t)(D >> 3) * 2048 + (size_t)(Dv >> 3) * 2048 + (size_t)(D >> 3) * 1024 + (size_t)(Dv >> 3) * 1024 + 2 * 16384;
-        const size_t smem64 = half64 * (x3 ? 2 : 1) + (x3 ? (size_t)(D >> 3) * (2048 + 1024) : 0);
-        if (q64 && smem64 <= 200 * 1024) {
-            static bool attr64 = false;
-            if (!attr64) {
-                if (cudaFuncSetAttribute(xattn_bwd_tc_q64_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024) != cudaSuccess ||
-                    cudaFuncSetAttribute(xattn_bwd_tc_q64_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024) != cudaSuccess) {
-                    cudaGetLastError();
-                    return NPF_ENOTSUP;
-                }
-                attr64 = true;
-            }
-            cudaMemsetAsync(dQ, 0, sizeof(float) * (size_t)B * Tq * H * D, st);   // dQ is accumulated over key blocks with atomics
-            dim3 grid((unsigned)cdiv(Tk, 128), (unsigned)H, (unsigned)B);
-            if (x3) xattn_bwd_tc_q64_kernel<3><<<grid, 256, smem64, st>>>(p);
-            else xattn_bwd_tc_q64_kernel<1><<<grid, 256, smem64, st>>>(p);
-            count_launch();
-            return check_launch("xattn_bwd_tc_q64_kernel");
-        }
-    }
-    const size_t half = (size_t)(2 * (D >> 3) + 2 * (Dv >> 3) + 32) * 2048;
-    const size_t smem = half * (x3 ? 2 : 1) + (x3 ? (size_t)2 * (D >> 3) * 2048 : 0);
+    const size_t half = (size_t)(D >> 3) * 2048 + (size_t)(Dv >> 3) * 2048 + (size_t)(D >> 3) * 1024 + (size_t)(Dv >> 3) * 1024 + 2 * 16384;
+    const size_t smem = half * (x3 ? 2 : 1) + (x3 ? (size_t)(D >> 3) * (2048 + 1024) : 0);
+    if (smem > 200 * 1024) return NPF_ENOTSUP;
     static bool attr = false;
     if (!attr) {
-        if (cudaFuncSetAttribute(xattn_bwd_tc_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024) != cudaSuccess ||
-            cudaFuncSetAttribute(xattn_bwd_tc_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024) != cudaSuccess) {
+        if (cudaFuncSetAttribute(xattn_bwd_tc_q64_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024) != cudaSuccess ||
+            cudaFuncSetAttribute(xattn_bwd_tc_q64_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024) != cudaSuccess) {
             cudaGetLastError();
             return NPF_ENOTSUP;
         }
         attr = true;
     }
-    if (smem > 200 * 1024) return NPF_ENOTSUP;
     cudaMemsetAsync(dQ, 0, sizeof(float) * (size_t)B * Tq * H * D, st);   // dQ is accumulated over key blocks with atomics
     dim3 grid((unsigned)cdiv(Tk, 128), (unsigned)H, (unsigned)B);
-    if (x3) xattn_bwd_tc_kernel<3><<<grid, 256, smem, st>>>(p);
-    else xattn_bwd_tc_kernel<1><<<grid, 256, smem, st>>>(p);
+    if (x3) xattn_bwd_tc_q64_kernel<3><<<grid, 256, smem, st>>>(p);
+    else xattn_bwd_tc_q64_kernel<1><<<grid, 256, smem, st>>>(p);
     count_launch();
-    return check_launch("xattn_bwd_tc_kernel");
+    return check_launch("xattn_bwd_tc_q64_kernel");
 }
 
 }  // namespace npf

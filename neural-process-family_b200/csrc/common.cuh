@@ -67,7 +67,6 @@ static inline long cdiv(long a, long b) { return (a + b - 1) / b; }
 // The early start is requested only while the stream is being captured into a CUDA graph (GraphedStep): there the kernel
 // order is the library's own, and no kernel that writes PARAMETERS (an optimizer step) can sit directly in front of a
 // kernel whose pre-wait prologue reads them.  Eager launches keep plain stream order (the wait is then a no-op).
-bool pdl_enabled();     // NPF_PDL=0 disables it everywhere
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 
@@ -78,7 +77,7 @@ static inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 b
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
-    const bool early = pdl_enabled() && cudaStreamIsCapturing(st, &cap) == cudaSuccess && cap == cudaStreamCaptureStatusActive;
+    const bool early = cudaStreamIsCapturing(st, &cap) == cudaSuccess && cap == cudaStreamCaptureStatusActive;
     attr[0].val.programmaticStreamSerializationAllowed = early ? 1 : 0;
     cfg.attrs = attr; cfg.numAttrs = 1;
     return cudaLaunchKernelEx(&cfg, kernel, KArgs(args)...);

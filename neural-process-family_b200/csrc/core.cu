@@ -1,6 +1,5 @@
 // Error plumbing and launch accounting for libnpf_b200.
 #include <stdarg.h>
-#include <stdlib.h>
 #include <string.h>
 
 #include <atomic>
@@ -20,11 +19,6 @@ void set_error(const char* fmt, ...) {
 }
 
 void count_launch(int n) { g_launches.fetch_add((unsigned long long)n, std::memory_order_relaxed); }
-
-bool pdl_enabled() {
-    static const bool on = [] { const char* e = getenv("NPF_PDL"); return !(e && e[0] == '0'); }();
-    return on;
-}
 
 static unsigned long long* g_trace = nullptr;
 unsigned long long* trace_buffer() { return g_trace; }

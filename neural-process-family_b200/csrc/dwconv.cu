@@ -9,8 +9,6 @@
 // staged float4 is read once per filter row instead of once per tap.  The same kernel with flipped filters and a
 // relu-mask epilogue is the data gradient; the filter gradient kernel uses the mirrored register scheme.
 // KW is a compile-time (padded) filter width in {9, 11, 19}; narrower filters are centred and zero-padded.
-#include <cstdlib>
-
 #include "common.cuh"
 
 namespace npf {
@@ -571,222 +569,9 @@ static int launch_dw1_bwd_fused(Dw1Params& p, float* dWt, float* dbias, int B, c
 }
 
 // ----------------------------------------------------------------------------------------------------------------
-// 2-D fast path (GridConvCNP / GridConvLNP, 32x32-ish images, k = 9 / 11): FFMA-bound (121 taps per output), so the
-// kernel is organised around register reuse.  CTA tile = 16 rows x 32 columns x 16 channels (halo tile in shared
-// memory, staged with batched 16-byte loads and shift-only index math); a thread owns 4 channels x 8 columns x TWO
-// output rows: every staged input row it reads (18 float4) feeds both output rows, and every filter row it reads
-// (KW float4) feeds 8 columns -> ~17 FFMA per shared-memory load, which balances the FFMA and LDS pipes.
-// ----------------------------------------------------------------------------------------------------------------
-constexpr int T2H = 16, T2W = 32, T2C = 16, T2Q = T2C / 4;
-
-template <int KW>
-__device__ __forceinline__ void stage_tile2d(float4* Xs, const float* __restrict__ X, long img, int H, int Wd, int C, int h0, int w0, int c0,
-                                             int kh, int relu_in, const float* scale, const float* shift) {
-    const int rows = T2H + kh - 1, cols = T2W + KW - 1;
-    const int ph = kh / 2, pw = KW / 2;
-    const int q = threadIdx.x & (T2Q - 1), cl = threadIdx.x >> 2;     // 128 threads: 4 quads x 32 column lanes
-    const int c = c0 + 4 * q;
-    const bool affine = relu_in && scale != nullptr;
-    float4 sc = make_float4(1.f, 1.f, 1.f, 1.f), sh = make_float4(0.f, 0.f, 0.f, 0.f);
-    if (affine) { sc = __ldg(reinterpret_cast<const float4*>(scale + c)); sh = __ldg(reinterpret_cast<const float4*>(shift + c)); }
-    const int gw_a = w0 + cl - pw, gw_b = w0 + 32 + cl - pw;
-    const bool a_ok = gw_a >= 0 && gw_a < Wd, b_ok = (32 + cl < cols) && gw_b >= 0 && gw_b < Wd;
-    for (int r0 = 0; r0 < rows; r0 += 4) {
-        float4 va[4], vb[4];
-#pragma unroll
-        for (int u = 0; u < 4; ++u) {
-            const int r = r0 + u, gh = h0 + r - ph;
-            va[u] = make_float4(0.f, 0.f, 0.f, 0.f); vb[u] = va[u];
-            if (r < rows && gh >= 0 && gh < H) {
-                const float* rowp = X + (img + (long)gh * Wd) * C + c;
-                if (a_ok) va[u] = __ldg(reinterpret_cast<const float4*>(rowp + (long)gw_a * C));
-                if (b_ok) vb[u] = __ldg(reinterpret_cast<const float4*>(rowp + (long)gw_b * C));
-            }
-        }
-#pragma unroll
-        for (int u = 0; u < 4; ++u) {
-            const int r = r0 + u, gh = h0 + r - ph;
-            if (r >= rows) continue;
-            const bool in_img = gh >= 0 && gh < H;
-            if (relu_in) {   // padding stays exactly 0: activation only on real pixels
-                if (in_img && a_ok) va[u] = act4(va[u], affine, sc, sh);
-                if (in_img && b_ok) vb[u] = act4(vb[u], affine, sc, sh);
-            }
-            Xs[((size_t)r * cols + cl) * T2Q + q] = va[u];
-            if (32 + cl < cols) Xs[((size_t)r * cols + 32 + cl) * T2Q + q] = vb[u];
-        }
-    }
-}
-
-template <int KW>
-__global__ void __launch_bounds__(128) dwconv2d_kernel(DwParams p) {
-    extern __shared__ __align__(16) float smem[];
-    const int rows = T2H + p.kh - 1, cols = T2W + KW - 1;
-    float4* Xs = reinterpret_cast<float4*>(smem);                 // [rows][cols][4]
-    float4* Ws = Xs + (size_t)rows * cols * T2Q;                  // [kh][KW][4]
-    const int tile = blockIdx.x;
-    const int h0 = (tile / p.tiles_w) * T2H, w0 = (tile % p.tiles_w) * T2W;
-    const int c0 = blockIdx.y * T2C;
-    const int b = blockIdx.z;
-    const int joff = (KW - p.kw) / 2;
-    const long img = (long)b * p.H * p.Wd;
-    for (int idx = threadIdx.x; idx < p.kh * KW * T2C; idx += 128) {
-        const int c = idx & (T2C - 1), j = (idx >> 4) % KW, i = (idx >> 4) / KW;
-        float v = 0.f;
-        const int jr = j - joff;
-        if (jr >= 0 && jr < p.kw && c0 + c < p.C) {
-            const int ii = p.flip ? p.kh - 1 - i : i, jj = p.flip ? p.kw - 1 - jr : jr;
-            v = __ldg(p.Wt + ((long)(c0 + c) * p.kh + ii) * p.kw + jj);
-        }
-        reinterpret_cast<float*>(Ws)[((size_t)i * KW + j) * T2C + c] = v;
-    }
-    stage_tile2d<KW>(Xs, p.X, img, p.H, p.Wd, p.C, h0, w0, c0, p.kh, p.relu_in, p.scale, p.shift);
-    __syncthreads();
-
-    const int q = threadIdx.x & 3, s = (threadIdx.x >> 2) & 3, rp = threadIdx.x >> 4;     // quad, 8-column strip, row pair
-    float4 acc[2][8];
-#pragma unroll
-    for (int r = 0; r < 2; ++r)
-#pragma unroll
-        for (int pp = 0; pp < 8; ++pp) acc[r][pp] = make_float4(0.f, 0.f, 0.f, 0.f);
-    for (int y = 0; y < p.kh + 1; ++y) {            // input rows 2*rp + y feed output rows 2*rp (tap row y) and 2*rp+1 (tap row y-1)
-        float4 xr[KW + 7];
-        const float4* xrow = Xs + ((size_t)(2 * rp + y) * cols + s * 8) * T2Q + q;
-#pragma unroll
-        for (int xc = 0; xc < KW + 7; ++xc) xr[xc] = xrow[(size_t)xc * T2Q];
-#pragma unroll
-        for (int r = 0; r < 2; ++r) {
-            const int i = y - r;
-            if (i < 0 || i >= p.kh) continue;
-            float4 w[KW];
-#pragma unroll
-            for (int j = 0; j < KW; ++j) w[j] = Ws[((size_t)i * KW + j) * T2Q + q];
-#pragma unroll
-            for (int j = 0; j < KW; ++j)
-#pragma unroll
-                for (int pp = 0; pp < 8; ++pp) acc[r][pp] = f4_fma(w[j], xr[pp + j], acc[r][pp]);
-        }
-    }
-    const int c = c0 + 4 * q;
-    float4 bv = make_float4(0.f, 0.f, 0.f, 0.f);
-    if (p.bias) bv = __ldg(reinterpret_cast<const float4*>(p.bias + c));
-    float4 sc = make_float4(1.f, 1.f, 1.f, 1.f), sh = make_float4(0.f, 0.f, 0.f, 0.f);
-    if (p.mask && p.scale) { sc = __ldg(reinterpret_cast<const float4*>(p.scale + c)); sh = __ldg(reinterpret_cast<const float4*>(p.shift + c)); }
-#pragma unroll
-    for (int r = 0; r < 2; ++r) {
-        const int gh = h0 + 2 * rp + r;
-        if (gh >= p.H) continue;
-#pragma unroll
-        for (int pp = 0; pp < 8; ++pp) {
-            const int gw = w0 + s * 8 + pp;
-            if (gw >= p.Wd) continue;
-            const long off = (img + (long)gh * p.Wd + gw) * p.C + c;
-            float4 v = make_float4(acc[r][pp].x + bv.x, acc[r][pp].y + bv.y, acc[r][pp].z + bv.z, acc[r][pp].w + bv.w);
-            if (p.mask) {
-                const float4 x = __ldg(reinterpret_cast<const float4*>(p.Xorig + off));
-                const float4 pre = make_float4(fmaf(sc.x, x.x, sh.x), fmaf(sc.y, x.y, sh.y), fmaf(sc.z, x.z, sh.z), fmaf(sc.w, x.w, sh.w));
-                v.x = pre.x > 0.f ? v.x * sc.x : 0.f; v.y = pre.y > 0.f ? v.y * sc.y : 0.f;
-                v.z = pre.z > 0.f ? v.z * sc.z : 0.f; v.w = pre.w > 0.f ? v.w * sc.w : 0.f;
-            }
-            if (p.res) {
-                const float4 rv = __ldg(reinterpret_cast<const float4*>(p.res + off));
-                v.x += rv.x; v.y += rv.y; v.z += rv.z; v.w += rv.w;
-            }
-            float4* out = reinterpret_cast<float4*>(p.Y + off);
-            if (p.accum) { const float4 o = *out; v.x += o.x; v.y += o.y; v.z += o.z; v.w += o.w; }
-            *out = v;
-        }
-    }
-}
-
-// 2-D filter gradient.  Thread = (channel quad, PAIR of filter rows, work split); per work item (output row, 8-column
-// strip) it reads the dY strip once (8 float4) and the two input rows (2 x 18 float4) -> 2 x 88 float4 FMAs.
-template <int KW>
-__global__ void __launch_bounds__(128) dwconv2d_wgrad_kernel(DwParams p, const float* __restrict__ dY, float* __restrict__ dWt) {
-    extern __shared__ __align__(16) float smem[];
-    const int rows = T2H + p.kh - 1, cols = T2W + KW - 1;
-    float4* Xs = reinterpret_cast<float4*>(smem);                       // [rows][cols][4]
-    float4* Gs = Xs + (size_t)rows * cols * T2Q;                        // [16][32][4]
-    float* dWs = reinterpret_cast<float*>(Gs + (size_t)T2H * T2W * T2Q);   // [kh][KW][16]
-    const int tile = blockIdx.x;
-    const int h0 = (tile / p.tiles_w) * T2H, w0 = (tile % p.tiles_w) * T2W;
-    const int c0 = blockIdx.y * T2C;
-    const int b = blockIdx.z;
-    const int joff = (KW - p.kw) / 2;
-    const long img = (long)b * p.H * p.Wd;
-    for (int idx = threadIdx.x; idx < p.kh * KW * T2C; idx += 128) dWs[idx] = 0.f;
-    stage_tile2d<KW>(Xs, p.X, img, p.H, p.Wd, p.C, h0, w0, c0, p.kh, p.relu_in, p.scale, p.shift);
-    {   // dY tile: 16 rows x 32 columns x 4 quads, zero outside the image
-        const int q = threadIdx.x & 3, cl = threadIdx.x >> 2;
-        for (int r0 = 0; r0 < T2H; r0 += 4) {
-            float4 v[4];
-#pragma unroll
-            for (int u = 0; u < 4; ++u) {
-                const int gh = h0 + r0 + u, gw = w0 + cl;
-                v[u] = make_float4(0.f, 0.f, 0.f, 0.f);
-                if (gh < p.H && gw < p.Wd) v[u] = __ldg(reinterpret_cast<const float4*>(dY + (img + (long)gh * p.Wd + gw) * p.C + c0 + 4 * q));
-            }
-#pragma unroll
-            for (int u = 0; u < 4; ++u) Gs[((size_t)(r0 + u) * T2W + cl) * T2Q + q] = v[u];
-        }
-    }
-    __syncthreads();
-    const int n_pairs = (p.kh + 1) / 2;                  // filter-row pairs
-    const int per_split = T2Q * n_pairs;                 // threads per work split
-    const int n_splits = 128 / per_split;
-    const int split = threadIdx.x / per_split, rem = threadIdx.x % per_split;
-    const int q = rem & 3, tp = rem >> 2;
-    if (split < n_splits) {
-        float4 acc[2][KW];
-#pragma unroll
-        for (int r = 0; r < 2; ++r)
-#pragma unroll
-            for (int j = 0; j < KW; ++j) acc[r][j] = make_float4(0.f, 0.f, 0.f, 0.f);
-        const int i0 = 2 * tp;
-        const bool second = i0 + 1 < p.kh;
-        for (int item = split; item < T2H * 4; item += n_splits) {     // (output row, strip)
-            const int h = item >> 2, st = item & 3;
-            float4 dy[8];
-#pragma unroll
-            for (int pp = 0; pp < 8; ++pp) dy[pp] = Gs[((size_t)h * T2W + st * 8 + pp) * T2Q + q];
-#pragma unroll
-            for (int r = 0; r < 2; ++r) {
-                if (r == 1 && !second) continue;
-                const float4* xrow = Xs + ((size_t)(h + i0 + r) * cols + st * 8) * T2Q + q;
-#pragma unroll
-                for (int xc = 0; xc < KW + 7; ++xc) {
-                    const float4 xv = xrow[(size_t)xc * T2Q];
-#pragma unroll
-                    for (int j = 0; j < KW; ++j) {
-                        const int pp = xc - j;
-                        if (pp >= 0 && pp < 8) acc[r][j] = f4_fma(dy[pp], xv, acc[r][j]);
-                    }
-                }
-            }
-        }
-#pragma unroll
-        for (int r = 0; r < 2; ++r) {
-            if (r == 1 && !second) continue;
-#pragma unroll
-            for (int j = 0; j < KW; ++j) {
-                float* d = dWs + ((size_t)(i0 + r) * KW + j) * T2C + 4 * q;
-                atomicAdd(d + 0, acc[r][j].x); atomicAdd(d + 1, acc[r][j].y); atomicAdd(d + 2, acc[r][j].z); atomicAdd(d + 3, acc[r][j].w);
-            }
-        }
-    }
-    __syncthreads();
-    for (int idx = threadIdx.x; idx < p.kh * KW * T2C; idx += 128) {
-        const int c = idx & (T2C - 1), j = (idx >> 4) % KW, ii = (idx >> 4) / KW;
-        const int jr = j - joff;
-        if (jr >= 0 && jr < p.kw && c0 + c < p.C) atomicAdd(dWt + ((long)(c0 + c) * p.kh + ii) * p.kw + jr, dWs[idx]);
-    }
-}
-
-// ----------------------------------------------------------------------------------------------------------------
-// 2-D path, second arrangement (round 2): a WARP owns one channel pair.  The kernel above keeps 4 channels x 8 columns x 2 rows per
-// thread and reads both the input window and the filter taps with LDS.128 from four different channel quads per warp: 40 shared-memory
-// wavefront groups per 176 float4 FMAs -- the shared-memory pipe (not the FMA pipe) is what saturates, at 30 % FMA utilisation.
-// Here every lane of a warp works on the SAME two channels (packed fp32x2: one FFMA2 per tap and pixel), so
+// 2-D fast path (GridConvCNP / GridConvLNP, 32x32-ish images, k = 9 / 11): FFMA-bound (121 taps per output), so the kernels are
+// organised around register reuse and the shared-memory pipe.  A WARP owns one channel pair, and every lane of it works on the SAME
+// two channels (packed fp32x2: one FFMA2 per tap and pixel), so
 //   * a filter tap is one address for the whole warp: LDS.128 broadcasts (two taps each, one wavefront);
 //   * a lane owns 8 rows x 4 columns of the 32 x 32 output tile (64 float2 accumulators); an input row segment (4 + KW - 1 pixels, 7
 //     LDS.128) is loaded ONCE and feeds every (output row, tap row) combination it belongs to: 44 FFMA2 per combination;
@@ -964,7 +749,7 @@ __global__ void __launch_bounds__(V2P * 32, 3) dwconv2d_v2_kernel(DwParams p) {
 }
 
 template <int KW>
-static int launch_dw2_v2(DwParams& p, int B, cudaStream_t st) {
+static int launch_dw2(DwParams& p, int B, cudaStream_t st) {
     constexpr int ROWS = V2T + KW - 1, PITCH = ROWS * 8 + 16;
     const size_t smem = (size_t)V2P * ROWS * PITCH + (size_t)V2P * KW * (KW + 1) * sizeof(float2);
     static bool attr = false;
@@ -975,10 +760,9 @@ static int launch_dw2_v2(DwParams& p, int B, cudaStream_t st) {
     count_launch();
     return check_launch("dwconv2d_v2_kernel");
 }
-static bool dw2_v2_on() { static const bool on = [] { const char* e = getenv("NPF_DWCONV2D_V2"); return !(e && e[0] == '0'); }(); return on; }
 
 // ----------------------------------------------------------------------------------------------------------------
-// 2-D filter gradient, second arrangement: dW[c,i,j] = sum_{b,h,w} dY[b,h,w,c] act(X)[b,h+i-p,w+j-p,c].
+// 2-D filter gradient: dW[c,i,j] = sum_{b,h,w} dY[b,h,w,c] act(X)[b,h+i-p,w+j-p,c].
 // A persistent CTA = 8 channels (4 pairs) x 3 groups of 4 filter rows = 12 warps; it walks a share of the images and keeps its
 // 4 x KW packed accumulators per lane IN REGISTERS for all of them: the cross-lane reduction (shuffles) and the atomics happen once per
 // CTA, not once per image.  Per image the act(X) halo tile and the dY tile are staged as channel-pair planes (the layout of
@@ -1132,7 +916,7 @@ __global__ void __launch_bounds__(V2P * WGG * 32, 1) dwconv2d_wgrad_v2_kernel(Dw
 }
 
 template <int KW>
-static int launch_dw2_wgrad_v2(DwParams& p, const float* dY, float* dWt, int B, cudaStream_t st) {
+static int launch_dw2_wgrad(DwParams& p, const float* dY, float* dWt, int B, cudaStream_t st) {
     constexpr int ROWS = V2T + KW - 1, PITCH = ROWS * 8 + 16;
     const size_t smem = (size_t)V2P * ROWS * PITCH + (size_t)V2P * V2T * (V2T * 8 + 16);
     static bool attr = false;
@@ -1150,33 +934,8 @@ static int launch_dw2_wgrad_v2(DwParams& p, const float* dY, float* dWt, int B, 
     return check_launch("dwconv2d_wgrad_v2_kernel");
 }
 
-static bool dw2_ok(int H, int C, int kh, int kw) { return H > 1 && C % T2C == 0 && kh == kw && kh <= 11; }
-
-template <int KW>
-static int launch_dw2(DwParams& p, int B, cudaStream_t st) {
-    if (dw2_v2_on() && p.C % (2 * V2P) == 0 && p.kh == p.kw) return launch_dw2_v2<KW>(p, B, st);
-    p.tiles_w = (int)cdiv(p.Wd, T2W);
-    const size_t smem = ((size_t)(T2H + p.kh - 1) * (T2W + KW - 1) * T2C + (size_t)p.kh * KW * T2C) * sizeof(float);
-    static bool attr = false;
-    if (!attr) { cudaFuncSetAttribute(dwconv2d_kernel<KW>, cudaFuncAttributeMaxDynamicSharedMemorySize, 110 * 1024); attr = true; }
-    dim3 grid((unsigned)(p.tiles_w * cdiv(p.H, T2H)), (unsigned)(p.C / T2C), (unsigned)B);
-    dwconv2d_kernel<KW><<<grid, 128, smem, st>>>(p);
-    count_launch();
-    return check_launch("dwconv2d_kernel");
-}
-
-template <int KW>
-static int launch_dw2_wgrad(DwParams& p, const float* dY, float* dWt, int B, cudaStream_t st) {
-    if (dw2_v2_on() && p.C % (2 * V2P) == 0 && p.kh == p.kw) return launch_dw2_wgrad_v2<KW>(p, dY, dWt, B, st);
-    p.tiles_w = (int)cdiv(p.Wd, T2W);
-    const size_t smem = ((size_t)(T2H + p.kh - 1) * (T2W + KW - 1) * T2C + (size_t)T2H * T2W * T2C + (size_t)p.kh * KW * T2C) * sizeof(float);
-    static bool attr = false;
-    if (!attr) { cudaFuncSetAttribute(dwconv2d_wgrad_kernel<KW>, cudaFuncAttributeMaxDynamicSharedMemorySize, 140 * 1024); attr = true; }
-    dim3 grid((unsigned)(p.tiles_w * cdiv(p.H, T2H)), (unsigned)(p.C / T2C), (unsigned)B);
-    dwconv2d_wgrad_kernel<KW><<<grid, 128, smem, st>>>(p, dY, dWt);
-    count_launch();
-    return check_launch("dwconv2d_wgrad_kernel");
-}
+// The 2-D kernels need C % (2 V2P) == 0 and a square filter; shapes outside dw2_ok run the generic dwconv_kernel.
+static bool dw2_ok(int H, int C, int kh, int kw) { return H > 1 && C % 16 == 0 && kh == kw && kh <= 11; }
 
 // sum[c] += sum_m X[m,c] ; sumsq[c] += sum_m X[m,c]^2   (also used for the conv bias gradient with sumsq == null)
 __global__ void __launch_bounds__(256) channel_stats_kernel(const float* __restrict__ X, const float* __restrict__ center, float* sum,

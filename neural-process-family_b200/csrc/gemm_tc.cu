@@ -18,8 +18,6 @@
 // Shapes covered: reduction dim <= 128 and output dim <= 256, both multiples of 16.  Anything else reports
 // NPF_ENOTSUP and the caller uses the fp32 FFMA kernel.
 #include <cstdio>
-#include <cstdlib>
-
 #include "tc_common.cuh"
 
 namespace npf {
@@ -772,255 +770,6 @@ __global__ void __launch_bounds__(kWsThreads, 1) mlp_chain_fwd_kernel(ChainParam
     if (warp == 0) tmem_dealloc(tmem, 256);
 }
 
-// ------------------------------------------------------------------------------------------------ fused backward 128 x 128 x 128
-// dX = (dY W) (.) (X > 0)   and   dW += dY^T X,  db += colsum(dY)   in ONE pass over dY and X (hot shape only).
-// The dY and X row tiles are staged once (SW128, bf16 hi/lo) and each is read by the tensor core two ways:
-//     dX tile  = dY[K-major view] x W^T[MN-major view of the row-staged W]                 -> TMEM accumulator t (double buffered)
-//     dW      += dY^T[MN-major view of the SAME dY bytes] x X[MN-major view of the X tile] -> one TMEM accumulator for the CTA
-//     db      += column sums of dY, taken by the producers from the registers the tile passes through (exact fp32)
-// so the separate weight-gradient kernel's second read of dY and X (2/5 of the backward traffic of a layer) disappears and
-// the relu mask comes from the staged X tile instead of a third global stream.  Roles: 16 producer warps (next tile held in
-// registers: 8 + 8 LDG.128 per thread in flight), 1 MMA warp, 8 epilogue warps.  TMEM: [0,256) dX x2, [256,384) dW.
-constexpr int kFbProdWarps = 16;
-constexpr int kFbEpiWarp0 = 17;
-constexpr int kFbThreads = (kFbEpiWarp0 + kWsEpiWarps) * 32;     // 800
-
-struct TcFusedParams {
-    const float* dY; long lddy;     // [M, 128]
-    const float* X; long ldx;       // [M, 128]  layer input (post-relu activations): wgrad operand and relu mask
-    const float* W; long ldw;       // [128 (n), 128 (k)]
-    float* dX; long lddx;           // [M, 128]
-    float* dW; long lddw;           // [128, 128]  +=
-    float* db;                      // [128] += or null
-    int M, n_tiles, rows_per_cta;
-    int relu_x, use_mask, w_vec, dw_vec;
-};
-
-__device__ __forceinline__ void fb_load_rows(float4 (&pre)[8], const float* __restrict__ g, long ld, int row_first, int rows_valid) {
-#pragma unroll
-    for (int i = 0; i < 8; ++i) {
-        pre[i] = (row_first + i < rows_valid) ? __ldg(reinterpret_cast<const float4*>(g)) : make_float4(0.f, 0.f, 0.f, 0.f);
-        g += ld;
-    }
-}
-
-template <int NSPLIT, bool HAS_MASK>
-__global__ void __launch_bounds__(kFbThreads, 1) linear_bwd_fused_kernel(TcFusedParams p) {
-    extern __shared__ __align__(1024) uint8_t smem_raw[];
-    __shared__ __align__(8) uint64_t bar_full, bar_empty, bar_mask, bar_dwfull, bar_tfull[2], bar_tempty[2];
-    __shared__ uint32_t tmem_slot;
-    __shared__ float s_db[128];
-
-    constexpr uint32_t kTile = 128u * 128u * 2u;                  // 32 KB
-    constexpr uint32_t kOp = (NSPLIT == 3 ? 2u : 1u) * kTile;     // one operand (hi [+ lo])
-    uint8_t* y_hi = smem_raw;            uint8_t* y_lo = y_hi + kTile;
-    uint8_t* x_hi = smem_raw + kOp;      uint8_t* x_lo = x_hi + kTile;
-    uint8_t* w_hi = smem_raw + 2 * kOp;  uint8_t* w_lo = w_hi + kTile;
-    float* scratch_all = reinterpret_cast<float*>(smem_raw + 3 * kOp);
-
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    if (warp == 0) tmem_alloc(&tmem_slot, 512);
-    if (tid == 32) {
-        mbar_init(&bar_full, kFbProdWarps * 32);
-        mbar_init(&bar_empty, 1);
-        mbar_init(&bar_mask, kWsEpiWarps * 32);
-        mbar_init(&bar_dwfull, 1);
-        for (int i = 0; i < 2; ++i) {
-            mbar_init(&bar_tfull[i], 1);
-            mbar_init(&bar_tempty[i], kWsEpiWarps * 32);
-        }
-    }
-    if (tid < 128) s_db[tid] = 0.f;
-
-    // producer / weight-staging geometry: warp w owns rows 8 w .. 8 w + 7, lane = float4 column
-    const uint32_t pchunk = (uint32_t)(lane >> 1) & 7u;
-    const uint32_t psoff = (uint32_t)(lane >> 4) * 16384u + (uint32_t)(warp * 8) * 128u + (uint32_t)(lane & 1) * 8u;
-    float4 py[8], px[8];
-    const int r_begin = blockIdx.x * p.rows_per_cta, r_end = min(p.M, r_begin + p.rows_per_cta);     // balanced contiguous row ranges
-    const int n_local = r_end > r_begin ? (r_end - r_begin + 127) >> 7 : 0;
-    pdl_trigger();
-    if (warp < kFbProdWarps) {
-        float4 wv[8];
-#pragma unroll
-        for (int i = 0; i < 8; ++i) {
-            const float* g = p.W + (long)(warp * 8 + i) * p.ldw + lane * 4;
-            if (p.w_vec) wv[i] = __ldg(reinterpret_cast<const float4*>(g));
-            else wv[i] = make_float4(__ldg(g), __ldg(g + 1), __ldg(g + 2), __ldg(g + 3));
-        }
-#pragma unroll
-        for (int i = 0; i < 8; ++i) cvt_store<NSPLIT>(wv[i], w_hi, w_lo, psoff + (uint32_t)i * 128u + ((pchunk ^ (uint32_t)i) << 4), 0);
-    }
-    fence_async_smem();
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem = tmem_slot;
-    pdl_wait();         // weights only so far; dY / X of the preceding kernels (and our dX / dW / db writes) from here on
-
-    if (warp < kFbProdWarps) {
-        // ------------------------------------------------------------------ producers
-        {
-            const int rv = min(128, r_end - r_begin);
-            fb_load_rows(py, p.dY + ((long)r_begin + warp * 8) * p.lddy + lane * 4, p.lddy, warp * 8, rv);
-            fb_load_rows(px, p.X + ((long)r_begin + warp * 8) * p.ldx + lane * 4, p.ldx, warp * 8, rv);
-            if (n_local > 1) {
-                prefetch_tile_l2(p.dY, p.lddy, (long)r_begin + 128, min(128, r_end - r_begin - 128), tid, kFbProdWarps * 32);
-                prefetch_tile_l2(p.X, p.ldx, (long)r_begin + 128, min(128, r_end - r_begin - 128), tid, kFbProdWarps * 32);
-            }
-        }
-        float4 dbs = make_float4(0.f, 0.f, 0.f, 0.f);
-        for (int it = 0; it < n_local; ++it) {
-#pragma unroll
-            for (int i = 0; i < 8; ++i) { dbs.x += py[i].x; dbs.y += py[i].y; dbs.z += py[i].z; dbs.w += py[i].w; }
-            if (it > 0) {
-                mbar_wait(&bar_empty, (it - 1) & 1);               // both MMA groups of the previous tile have read the stage
-                if (HAS_MASK) mbar_wait(&bar_mask, (it - 1) & 1);  // and the epilogue has taken its relu mask from it
-            }
-#pragma unroll
-            for (int i = 0; i < 8; ++i) {
-                const uint32_t off = psoff + (uint32_t)i * 128u + ((pchunk ^ (uint32_t)i) << 4);
-                cvt_store<NSPLIT>(py[i], y_hi, y_lo, off, 0);
-                cvt_store<NSPLIT>(px[i], x_hi, x_lo, off, p.relu_x);
-            }
-            fence_async_smem();
-            mbar_arrive(&bar_full);
-            if (it + 1 < n_local) {
-                const int nrow = r_begin + (it + 1) * 128, rv = min(128, r_end - nrow);
-                fb_load_rows(py, p.dY + ((long)nrow + warp * 8) * p.lddy + lane * 4, p.lddy, warp * 8, rv);
-                fb_load_rows(px, p.X + ((long)nrow + warp * 8) * p.ldx + lane * 4, p.ldx, warp * 8, rv);
-                if (it + 2 < n_local) {
-                    prefetch_tile_l2(p.dY, p.lddy, (long)nrow + 128, min(128, r_end - nrow - 128), tid, kFbProdWarps * 32);
-                    prefetch_tile_l2(p.X, p.ldx, (long)nrow + 128, min(128, r_end - nrow - 128), tid, kFbProdWarps * 32);
-                }
-            }
-        }
-        if (p.db) {                                                  // bias gradient: warps -> smem -> one global atomic per column
-            atomicAdd(&s_db[lane * 4 + 0], dbs.x); atomicAdd(&s_db[lane * 4 + 1], dbs.y);
-            atomicAdd(&s_db[lane * 4 + 2], dbs.z); atomicAdd(&s_db[lane * 4 + 3], dbs.w);
-            asm volatile("bar.sync 1, %0;" ::"n"(kFbProdWarps * 32) : "memory");
-            if (tid < 128) atomicAdd(p.db + tid, s_db[tid]);
-        }
-    } else if (warp == kFbProdWarps) {
-        // ------------------------------------------------------------------ MMA issuer
-        if (lane == 0) {
-            const uint32_t idesc_dx = make_idesc(128, 128, 0, 1);    // A = dY K-major, B = W^T (MN-major view)
-            const uint32_t idesc_dw = make_idesc(128, 128, 1, 1);    // A = dY^T, B = X: both MN-major views (reduction over rows)
-            const uint32_t sy_hi = smem_u32(y_hi), sy_lo = smem_u32(y_lo), sx_hi = smem_u32(x_hi), sx_lo = smem_u32(x_lo);
-            const uint32_t sw_hi = smem_u32(w_hi), sw_lo = smem_u32(w_lo);
-            const uint32_t d_dw = tmem + 256u;
-            for (int it = 0; it < n_local; ++it) {
-                const int t = it & 1;
-                mbar_wait(&bar_full, it & 1);
-                mbar_wait(&bar_tempty[t], ((it >> 1) & 1) ^ 1);
-                tc_fence_after();
-                const uint32_t d_dx = tmem + (uint32_t)t * 128u;
-#pragma unroll
-                for (int ks = 0; ks < 8; ++ks) {                     // reduction over n
-                    const uint32_t ao = (uint32_t)(ks >> 2) * 16384u + (uint32_t)(ks & 3) * 32u;
-                    const uint64_t a_h = make_desc_sw128(sy_hi + ao, 16, 1024), b_h = make_desc_sw128(sw_hi + ks * 2048u, 16384, 1024);
-                    umma_bf16(d_dx, a_h, b_h, idesc_dx, ks ? 1u : 0u);
-                    if (NSPLIT == 3) {
-                        umma_bf16(d_dx, a_h, make_desc_sw128(sw_lo + ks * 2048u, 16384, 1024), idesc_dx, 1);
-                        umma_bf16(d_dx, make_desc_sw128(sy_lo + ao, 16, 1024), b_h, idesc_dx, 1);
-                    }
-                }
-                umma_commit(&bar_tfull[t]);
-#pragma unroll
-                for (int ks = 0; ks < 8; ++ks) {                     // reduction over the 128 rows of the tile
-                    const uint32_t acc = (it | ks) ? 1u : 0u;
-                    const uint64_t a_h = make_desc_sw128(sy_hi + ks * 2048u, 16384, 1024), b_h = make_desc_sw128(sx_hi + ks * 2048u, 16384, 1024);
-                    umma_bf16(d_dw, a_h, b_h, idesc_dw, acc);
-                    if (NSPLIT == 3) {
-                        const uint64_t a_l = make_desc_sw128(sy_lo + ks * 2048u, 16384, 1024);
-                        umma_bf16(d_dw, a_h, make_desc_sw128(sx_lo + ks * 2048u, 16384, 1024), idesc_dw, 1);
-                        umma_bf16(d_dw, a_l, b_h, idesc_dw, 1);
-                    }
-                }
-                umma_commit(&bar_empty);
-            }
-            umma_commit(&bar_dwfull);
-        }
-    } else {
-        // ------------------------------------------------------------------ epilogue
-        const int e = warp - kFbEpiWarp0;
-        const int lane_base = 32 * (warp & 3);
-        const int col_base = (e >> 2) * 64;
-        float* scratch = scratch_all + e * (32 * kWsScratchLd);
-        const int r_in = lane >> 2, c4 = (lane & 3) * 4;
-        for (int it = 0; it < n_local; ++it) {
-            const int t = it & 1;
-            const int m0 = r_begin + it * 128 + lane_base;
-            mbar_wait(&bar_tfull[t], (it >> 1) & 1);
-            tc_fence_after();
-            unsigned long long mbits = ~0ull;
-            if (HAS_MASK) {          // relu mask of this thread's 16 float4 outputs, from the staged (relu'd) X tile: bf16 > 0 <=> int16 > 0
-                mbits = 0ull;
-#pragma unroll
-                for (int ch = 0; ch < 4; ++ch) {
-#pragma unroll
-                    for (int j = 0; j < 4; ++j) {
-                        const int r = lane_base + j * 8 + r_in, c = col_base + ch * 16 + c4;
-                        const uint2 xb = *reinterpret_cast<const uint2*>(x_hi + (uint32_t)(c >> 6) * 16384u + (uint32_t)r * 128u +
-                                                                       ((((uint32_t)(c & 63) >> 3) ^ (uint32_t)(r & 7)) << 4) + (uint32_t)(c & 7) * 2u);
-                        const unsigned long long b4 = ((short)(xb.x & 0xFFFFu) > 0 ? 1ull : 0ull) | ((short)(xb.x >> 16) > 0 ? 2ull : 0ull) |
-                                                      ((short)(xb.y & 0xFFFFu) > 0 ? 4ull : 0ull) | ((short)(xb.y >> 16) > 0 ? 8ull : 0ull);
-                        mbits |= b4 << ((ch * 4 + j) * 4);
-                    }
-                }
-                mbar_arrive(&bar_mask);
-            }
-#pragma unroll 1
-            for (int ch = 0; ch < 4; ++ch) {
-                const int c0 = col_base + ch * 16;
-                float v[16];
-                tmem_ld16(tmem + ((uint32_t)lane_base << 16) + (uint32_t)(t * 128 + c0), v);
-                if (ch == 3) {
-                    tc_fence_before();
-                    mbar_arrive(&bar_tempty[t]);
-                }
-#pragma unroll
-                for (int j = 0; j < 16; j += 4)
-                    *reinterpret_cast<float4*>(scratch + lane * kWsScratchLd + j) = make_float4(v[j], v[j + 1], v[j + 2], v[j + 3]);
-                __syncwarp();
-#pragma unroll
-                for (int j = 0; j < 4; ++j) {
-                    const int r = j * 8 + r_in;
-                    const int row = m0 + r;
-                    if (row < r_end) {
-                        float4 x = *reinterpret_cast<const float4*>(scratch + r * kWsScratchLd + c4);
-                        if (HAS_MASK) {
-                            const unsigned b4 = (unsigned)(mbits >> ((ch * 4 + j) * 4));
-                            x.x = (b4 & 1u) ? x.x : 0.f; x.y = (b4 & 2u) ? x.y : 0.f; x.z = (b4 & 4u) ? x.z : 0.f; x.w = (b4 & 8u) ? x.w : 0.f;
-                        }
-                        *reinterpret_cast<float4*>(p.dX + (long)row * p.lddx + c0 + c4) = x;
-                    }
-                }
-                __syncwarp();
-            }
-        }
-        // ---- flush of the CTA's weight / bias gradient: thread = row n of dW, 64 columns per warp
-        mbar_wait(&bar_dwfull, 0);
-        tc_fence_after();
-        const int n = lane_base + lane;
-#pragma unroll 1
-        for (int ch = 0; ch < 4; ++ch) {
-            const int c0 = col_base + ch * 16;
-            float v[16];
-            tmem_ld16(tmem + ((uint32_t)lane_base << 16) + (uint32_t)(256 + c0), v);
-            float* d = p.dW + (long)n * p.lddw + c0;
-            if (p.dw_vec) {
-#pragma unroll
-                for (int j = 0; j < 16; j += 4) atomicAdd(reinterpret_cast<float4*>(d + j), make_float4(v[j], v[j + 1], v[j + 2], v[j + 3]));
-            } else {
-                atomic_add16(d, v);
-            }
-        }
-    }
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 0) tmem_dealloc(tmem, 512);
-}
-
 // ------------------------------------------------------------------------------------------------ weight gradient
 // dW[n, k] += sum_m dY[m, n] X[m, k].  MMA shape M = N_out (rows of dW, <= 128 -> padded to 128), N = K_out, K = rows m.
 // Both operands MN-major, no swizzle: element (mn, k) at byte (k/8)*LBO + (mn/8)*128 + (k%8)*16 + (mn%8)*2,
@@ -1312,15 +1061,35 @@ int linear_bwd_data_tc(const float* dY, int lddy, const float* W, int ldw, float
 
 
 // ------------------------------------------------------------------------------------------------ fused backward, 64-row tiles
-// Same mathematics as linear_bwd_fused_kernel, re-cut so that the operand stage fits TWICE in shared memory (x3: 2 x 64 KB +
-// 64 KB of weights): with 128-row tiles a single stage forces "convert+store tile i+1" to wait for "multiply tile i"
-// (14 k cycles per tile measured, against 8.7 k of HBM time).  With 64-row tiles the tensor-core M dimension is kept at
-// 128 by computing the TRANSPOSED data gradient:
+// dX = (dY W) (.) (X > 0)   and   dW += dY^T X,  db += colsum(dY)   in ONE pass over dY and X (hot shape only).
+// The dY and X row tiles are staged once (SW128, bf16 hi/lo) and each is read by the tensor core two ways:
 //     dX^T[k, m] = sum_n W[n, k] dY[m, n]      A = W^T (MN-major view of the row-staged W),  B = dY tile (K-major),  N = 64
-//     dW[n, k]  += sum_m dY[m, n] X[m, k]      A = dY^T, B = X (MN-major views), 4 k-steps of 16 rows
-// The accumulator then has k on the TMEM lanes and the tile's rows on the columns, so an epilogue thread owns ONE column k
-// of dX and every register it reads is one row: a warp store covers 128 contiguous bytes without any shared-memory
-// transpose, and the relu mask is a 2-byte read of the staged X tile.  Producers keep TWO tiles in flight in registers.
+//     dW[n, k]  += sum_m dY[m, n] X[m, k]      A = dY^T, B = X (MN-major views of the same bytes), 4 k-steps of 16 rows
+//     db        += column sums of dY, taken by the producers from the registers the tile passes through (exact fp32)
+// so a separate weight-gradient kernel's second read of dY and X (2/5 of the backward traffic of a layer) is not needed and
+// the relu mask comes from the staged X tile instead of a third global stream.
+// Tiles are 64 rows so that the operand stage fits TWICE in shared memory (x3: 2 x 64 KB + 64 KB of weights): a 128-row
+// stage fits only once, and "convert+store tile i+1" then waits for "multiply tile i" (14 k cycles per tile measured, against
+// 8.7 k of HBM time).  The tensor-core M dimension is kept at 128 by computing the data gradient TRANSPOSED: the accumulator
+// has k on the TMEM lanes and the tile's rows on the columns, so an epilogue thread owns ONE column k of dX and every register
+// it reads is one row: a warp store covers 128 contiguous bytes without any shared-memory transpose, and the relu mask is a
+// 2-byte read of the staged X tile.  Roles: 16 producer warps (TWO tiles in flight in registers), 1 MMA warp, 8 epilogue
+// warps.  TMEM: [0,128) dX^T x2, [128,256) dW.
+constexpr int kFbProdWarps = 16;
+constexpr int kFbEpiWarp0 = 17;
+constexpr int kFbThreads = (kFbEpiWarp0 + kWsEpiWarps) * 32;     // 800
+
+struct TcFusedParams {
+    const float* dY; long lddy;     // [M, 128]
+    const float* X; long ldx;       // [M, 128]  layer input (post-relu activations): wgrad operand and relu mask
+    const float* W; long ldw;       // [128 (n), 128 (k)]
+    float* dX; long lddx;           // [M, 128]
+    float* dW; long lddw;           // [128, 128]  +=
+    float* db;                      // [128] += or null
+    int M, n_tiles, rows_per_cta;
+    int relu_x, use_mask, w_vec, dw_vec;
+};
+
 #ifndef F64_DEPTH
 #define F64_DEPTH 1
 #endif
@@ -1562,11 +1331,10 @@ __global__ void __launch_bounds__(kFbThreads, 1) linear_bwd_fused64_kernel(TcFus
 // then runs the two separate kernels).
 template <int NSPLIT>
 static int launch_fused(TcFusedParams& p, cudaStream_t st) {
-    const size_t smem = (size_t)3 * (NSPLIT == 3 ? 2 : 1) * 32768 + (size_t)kWsEpiWarps * 32 * kWsScratchLd * sizeof(float);
     static bool attr = false;
     if (!attr) {
-        if (cudaFuncSetAttribute(linear_bwd_fused_kernel<NSPLIT, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 224 * 1024) != cudaSuccess ||
-            cudaFuncSetAttribute(linear_bwd_fused_kernel<NSPLIT, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 224 * 1024) != cudaSuccess) {
+        if (cudaFuncSetAttribute(linear_bwd_fused64_kernel<NSPLIT, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 224 * 1024) != cudaSuccess ||
+            cudaFuncSetAttribute(linear_bwd_fused64_kernel<NSPLIT, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 224 * 1024) != cudaSuccess) {
             cudaGetLastError();
             return NPF_ENOTSUP;
         }
@@ -1576,27 +1344,11 @@ static int launch_fused(TcFusedParams& p, cudaStream_t st) {
     int grid = p.n_tiles < kNumSMs ? p.n_tiles : kNumSMs;
     p.rows_per_cta = (int)(cdiv(cdiv(p.M, grid), 8) * 8);
     grid = (int)cdiv(p.M, p.rows_per_cta);
-    static const bool v64 = getenv("NPF_FUSED64") ? atoi(getenv("NPF_FUSED64")) != 0 : true;
-    if (v64) {      // 64-row tiles, two operand stages (no epilogue scratch)
-        static bool attr64 = false;
-        if (!attr64) {
-            if (cudaFuncSetAttribute(linear_bwd_fused64_kernel<NSPLIT, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 224 * 1024) != cudaSuccess ||
-                cudaFuncSetAttribute(linear_bwd_fused64_kernel<NSPLIT, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 224 * 1024) != cudaSuccess) {
-                cudaGetLastError();
-                return NPF_ENOTSUP;
-            }
-            attr64 = true;
-        }
-        const size_t smem64 = (size_t)(NSPLIT == 3 ? 2 : 1) * (4 * 16384 + 32768);
-        if (p.use_mask) launch_pdl(linear_bwd_fused64_kernel<NSPLIT, true>, grid, kFbThreads, smem64, st, p);
-        else launch_pdl(linear_bwd_fused64_kernel<NSPLIT, false>, grid, kFbThreads, smem64, st, p);
-        count_launch();
-        return check_launch("linear_bwd_fused64_kernel");
-    }
-    if (p.use_mask) launch_pdl(linear_bwd_fused_kernel<NSPLIT, true>, grid, kFbThreads, smem, st, p);
-    else launch_pdl(linear_bwd_fused_kernel<NSPLIT, false>, grid, kFbThreads, smem, st, p);
+    const size_t smem = (size_t)(NSPLIT == 3 ? 2 : 1) * (4 * 16384 + 32768);      // two 64-row dY + X stages, the weights
+    if (p.use_mask) launch_pdl(linear_bwd_fused64_kernel<NSPLIT, true>, grid, kFbThreads, smem, st, p);
+    else launch_pdl(linear_bwd_fused64_kernel<NSPLIT, false>, grid, kFbThreads, smem, st, p);
     count_launch();
-    return check_launch("linear_bwd_fused_kernel");
+    return check_launch("linear_bwd_fused64_kernel");
 }
 
 int linear_bwd_fused_tc(const float* dY, int lddy, const float* X, int ldx, const float* W, int ldw, float* dX, int lddx, float* dW,

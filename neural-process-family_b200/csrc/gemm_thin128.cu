@@ -11,8 +11,6 @@
 // instruction), the narrow side lives in registers (compile-time R / J), rows are processed kRows at a time so that kRows
 // independent 16-byte accesses per thread are in flight, and the CTA's column sums go through shared memory before ONE
 // global atomic per entry.  Grids are persistent (a few CTAs per SM): no per-row index arithmetic, no divisions.
-#include <cstdlib>
-
 #include "common.cuh"
 #include "gemm_thin.cuh"
 
@@ -268,8 +266,7 @@ int thin128_in_bwd(const float* dY, long lddy, const float* X, long ldx, const f
     Thin128Params p{};
     p.dY = dY; p.lddy = lddy; p.X = X; p.ldx = ldx; p.W = W; p.ldw = ldw; p.Y = dX; p.ldy = lddx; p.dW = dW; p.lddw = lddw; p.db = db;
     p.M = M; p.relu_in = relu_in;
-    static const int per_sm = [] { const char* e = getenv("NPF_THIN_IN_BWD_CTAS"); const int v = e ? atoi(e) : 0; return v >= 1 && v <= 8 ? v : 2; }();
-    const unsigned grid = t128_grid(M, per_sm);
+    const unsigned grid = t128_grid(M, 2);
     NPF_T128_SWITCH(R, thin_in128_bwd_kernel, grid)
     count_launch();
     return check_launch("thin_in128_bwd_kernel");

@@ -15,10 +15,8 @@
 //     buffered in TMEM).  The product is issued TRANSPOSED, Y^T = Wpw . O^T (both images are 128-column K-major, so they just swap
 //     roles): TMEM lane = output channel, column = tile row, and the 8 epilogue warps store 32 consecutive channels of a row straight
 //     from their tcgen05.ld registers -- no shared-memory transpose.  With the rows as the N extent of the MMA the tile may be 96 rows
-//     high (chosen when it leaves fewer rows on the busiest CTA).  NPF_RB_FWD_T = 0 keeps the row-major product (+ transpose),
-//     = 2 reads Wpw from TMEM (tcgen05.mma with a TMEM A operand; measured slower).
+//     high (chosen when it leaves fewer rows on the busiest CTA).
 // HBM sees X once (+ 2p / 128 halo re-reads out of L2) and Y once.
-#include <cstdlib>
 #include <type_traits>
 
 #include "tc_common.cuh"
@@ -33,7 +31,6 @@ constexpr int kRbThreads = (kRbEpiWarp0 + kRbEpi) * 32;       // 800
 constexpr int kRbMaxPad = 9;                                   // k <= 19
 constexpr int kRbRawRows = 128 + 2 * kRbMaxPad;                // 146
 constexpr uint32_t kRbTile = 128u * 128u * 2u;                 // one bf16 128 x 128 image: 32 KB
-constexpr int kRbScratchLd = 20;
 
 struct RbFwdParams {
     const float* X;      // [B, L, 128]
@@ -44,7 +41,6 @@ struct RbFwdParams {
     float* O;            // [B, L, 128] or null
     float* Y;            // [B, L, 128]
     int B, L, n_lt, n_tiles;
-    int transposed;      // Y^T = Wpw . O^T (thread = output channel in the epilogue: rows stored straight from registers)
     unsigned long long* trace;      // diagnostics (npf_debug_set_trace)
 };
 
@@ -57,7 +53,7 @@ __device__ __forceinline__ uint32_t rb_img_off(uint32_t row, uint32_t col) {
 }
 __device__ __forceinline__ void rb_prod_sync() { asm volatile("bar.sync 1, %0;" ::"n"(kRbProd * 32) : "memory"); }
 
-// TR = rows per tile: 128, or (transposed product only: the rows are then the N extent of the MMA) 96 when that splits the tiles more
+// TR = rows per tile: 128, or (the rows are the N extent of the MMA) 96 when that splits the tiles more
 // evenly over the CTAs -- config 2: 768 tiles of 128 rows are 6 rounds on 148 SMs (768 rows on the critical CTA), 1024 tiles of 96 are 7 (672).
 template <int KW, int TR>
 __global__ void __launch_bounds__(kRbThreads, 1) resblock1d_fwd_kernel(RbFwdParams p) {
@@ -70,16 +66,14 @@ __global__ void __launch_bounds__(kRbThreads, 1) resblock1d_fwd_kernel(RbFwdPara
     __shared__ uint32_t tmem_slot;
     __shared__ __align__(16) float s_bias[128];
 
-    uint8_t* a_hi = smem_raw;                                   // O image (A operand)
+    uint8_t* a_hi = smem_raw;                                   // O image (B operand of Y^T = Wpw . O^T)
     uint8_t* a_lo = a_hi + kRbTile;
-    uint8_t* b_hi = smem_raw + 2 * kRbTile;                     // pointwise weights (B operand)
+    uint8_t* b_hi = smem_raw + 2 * kRbTile;                     // pointwise weights (A operand)
     uint8_t* b_lo = b_hi + kRbTile;
     float* raw = reinterpret_cast<float*>(smem_raw + 4 * kRbTile);          // [RAW][128] fp32
-    float* scratch_all = raw + kRbRawRows * 128;
 
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const uint32_t tmem_cols = p.transposed == 2 ? 512u : 256u;    // + 128 columns of pointwise weights when A is read from TMEM
-    if (warp == 0) tmem_alloc(&tmem_slot, tmem_cols);
+    if (warp == 0) tmem_alloc(&tmem_slot, 256);
     if (tid == 32) {
         mbar_init(&bar_raw, 1);
         mbar_init(&bar_afull, kRbProd * 32);
@@ -114,32 +108,6 @@ __global__ void __launch_bounds__(kRbThreads, 1) resblock1d_fwd_kernel(RbFwdPara
     __syncthreads();
     tc_fence_after();
     const uint32_t tmem = tmem_slot;
-    if (p.transposed == 2) {
-        // pointwise weights as the TMEM-resident A operand of Y^T = Wpw . O^T: lane n = row n of Wpw [out, in] (K-major over `in`),
-        // hi at columns [256, 320), lo at [320, 384); two consecutive `in` entries per 32-bit column
-        if (warp < 4) {
-            const float* wr = p.wpw + (long)(32 * warp + lane) * 128;
-            const uint32_t tw = tmem + ((uint32_t)(32 * warp) << 16) + 256u;
-#pragma unroll 1
-            for (int cc = 0; cc < 4; ++cc) {
-                uint32_t hi[16], lo[16];
-#pragma unroll
-                for (int q = 0; q < 8; ++q) {
-                    const float4 v = __ldg(reinterpret_cast<const float4*>(wr + cc * 32) + q);
-                    const uint32_t h01 = pack_bf16(v.x, v.y), h23 = pack_bf16(v.z, v.w);
-                    hi[2 * q] = h01; hi[2 * q + 1] = h23;
-                    lo[2 * q] = pack_bf16(v.x - __uint_as_float(h01 << 16), v.y - __uint_as_float(h01 & 0xFFFF0000u));
-                    lo[2 * q + 1] = pack_bf16(v.z - __uint_as_float(h23 << 16), v.w - __uint_as_float(h23 & 0xFFFF0000u));
-                }
-                tmem_st16(tw + (uint32_t)(cc * 16), hi);
-                tmem_st16(tw + 64u + (uint32_t)(cc * 16), lo);
-            }
-            tmem_st_wait();
-        }
-        tc_fence_before();
-        __syncthreads();
-        tc_fence_after();
-    }
     pdl_wait();
 
     if (warp < kRbProd) {
@@ -222,7 +190,7 @@ __global__ void __launch_bounds__(kRbThreads, 1) resblock1d_fwd_kernel(RbFwdPara
     } else if (warp == kRbMmaWarp) {
         // ------------------------------------------------------------------ MMA issuer
         if (lane == 0) {
-            const uint32_t idesc = make_idesc(128, TR, 0, 0);          // N = TR < 128 only in the transposed orientations (launch_rb_fwd)
+            const uint32_t idesc = make_idesc(128, TR, 0, 0);
             const uint64_t da_h = rb_desc_sw128(smem_u32(a_hi), 16, 1024), da_l = rb_desc_sw128(smem_u32(a_lo), 16, 1024);
             const uint64_t db_h = rb_desc_sw128(smem_u32(b_hi), 16, 1024), db_l = rb_desc_sw128(smem_u32(b_lo), 16, 1024);
             int it = 0;
@@ -238,20 +206,10 @@ __global__ void __launch_bounds__(kRbThreads, 1) resblock1d_fwd_kernel(RbFwdPara
                 for (int ks = 0; ks < 8; ++ks) {
                     const uint32_t ao = (uint32_t)(ks >> 2) * 16384u + (uint32_t)(ks & 3) * 32u;
                     const uint64_t a_h = desc_adv(da_h, ao), b_h = desc_adv(db_h, ao);
-                    if (p.transposed == 2) {  // A = Wpw from TMEM (8 columns per 16-wide k-slice): only the O image is read from shared memory
-                        const uint32_t ta = tmem + 256u + (uint32_t)ks * 8u;
-                        umma_bf16_ts(d, ta, a_h, idesc, ks ? 1u : 0u);
-                        umma_bf16_ts(d, ta + 64u, a_h, idesc, 1);
-                        umma_bf16_ts(d, ta, desc_adv(da_l, ao), idesc, 1);
-                    } else if (p.transposed) {      // both images are 128 x 128 K-major: swapping the operands transposes the product
-                        umma_bf16(d, b_h, a_h, idesc, ks ? 1u : 0u);
-                        umma_bf16(d, desc_adv(db_l, ao), a_h, idesc, 1);
-                        umma_bf16(d, b_h, desc_adv(da_l, ao), idesc, 1);
-                    } else {
-                        umma_bf16(d, a_h, b_h, idesc, ks ? 1u : 0u);
-                        umma_bf16(d, a_h, desc_adv(db_l, ao), idesc, 1);
-                        umma_bf16(d, desc_adv(da_l, ao), b_h, idesc, 1);
-                    }
+                    // Y^T = Wpw . O^T: both images are 128 x 128 K-major, so swapping the operands transposes the product
+                    umma_bf16(d, b_h, a_h, idesc, ks ? 1u : 0u);
+                    umma_bf16(d, desc_adv(db_l, ao), a_h, idesc, 1);
+                    umma_bf16(d, b_h, desc_adv(da_l, ao), idesc, 1);
                 }
                 umma_commit(&bar_aempty);
                 umma_commit(&bar_tfull[t]);
@@ -259,75 +217,44 @@ __global__ void __launch_bounds__(kRbThreads, 1) resblock1d_fwd_kernel(RbFwdPara
             }
         }
     } else {
-        // ------------------------------------------------------------------ epilogue: TMEM -> + bias -> coalesced rows of Y
+        // ------------------------------------------------------------------ epilogue: TMEM -> + bias -> rows of Y
+        // TMEM lane = output channel, columns = the tile's rows: a warp stores 32 consecutive channels of one row
         const int e = warp - kRbEpiWarp0;
         const int lane_base = 32 * (warp & 3);
-        const int col_base = (e >> 2) * 64;
-        float* scratch = scratch_all + e * (32 * kRbScratchLd);
-        const int r_in = lane >> 2, c4 = (lane & 3) * 4;
         int it = 0;
         for (int g = g0; g < g1; ++g, ++it) {
             const int t = it & 1;
             const int b = g / p.n_lt, l0 = (g - b * p.n_lt) * TR;
-            const int rows_ok = min(TR, p.L - l0) - lane_base;         // rows [0, rows_ok) of this warp's 32 exist
-            float* yb = p.Y + ((long)b * p.L + l0 + lane_base) * 128;
             if (e == 0 && lane == 0) trace_ev(p.trace, 2, 1);
             mbar_wait(&bar_tfull[t], (uint32_t)(it >> 1) & 1u);
             tc_fence_after();
             if (e == 0 && lane == 0) trace_ev(p.trace, 2, 2);
-            if (p.transposed) {        // TMEM lane = output channel, columns = the tile's rows: a warp stores 32 consecutive channels of one row
-                const float bias = s_bias[lane_base + lane];
-                const int rows_tile = min(TR, p.L - l0);
-                float* yc = p.Y + ((long)b * p.L + l0) * 128 + lane_base + lane;
+            const float bias = s_bias[lane_base + lane];
+            const int rows_tile = min(TR, p.L - l0);
+            float* yc = p.Y + ((long)b * p.L + l0) * 128 + lane_base + lane;
 #pragma unroll 1
-                for (int ch = 0; ch < TR / 32; ++ch) {              // this warp's half of the tile's rows, 16 at a time
-                    const int r0 = (e >> 2) * (TR / 2) + ch * 16;
-                    float v[16];
-                    tmem_ld16(tmem + ((uint32_t)lane_base << 16) + (uint32_t)(t * 128 + r0), v);
-                    if (ch == TR / 32 - 1) {
-                        tc_fence_before();
-                        mbar_arrive(&bar_tempty[t]);
-                    }
-#pragma unroll
-                    for (int j = 0; j < 16; ++j)
-                        if (r0 + j < rows_tile) yc[(long)(r0 + j) * 128] = v[j] + bias;
-                }
-                continue;
-            }
-#pragma unroll 1
-            for (int ch = 0; ch < 4; ++ch) {
-                const int c0 = col_base + ch * 16;
+            for (int ch = 0; ch < TR / 32; ++ch) {              // this warp's half of the tile's rows, 16 at a time
+                const int r0 = (e >> 2) * (TR / 2) + ch * 16;
                 float v[16];
-                tmem_ld16(tmem + ((uint32_t)lane_base << 16) + (uint32_t)(t * 128 + c0), v);
-                if (ch == 3) {
+                tmem_ld16(tmem + ((uint32_t)lane_base << 16) + (uint32_t)(t * 128 + r0), v);
+                if (ch == TR / 32 - 1) {
                     tc_fence_before();
                     mbar_arrive(&bar_tempty[t]);
                 }
 #pragma unroll
-                for (int j = 0; j < 16; j += 4) *reinterpret_cast<float4*>(scratch + lane * kRbScratchLd + j) = make_float4(v[j], v[j + 1], v[j + 2], v[j + 3]);
-                __syncwarp();
-                const float4 bb = *reinterpret_cast<const float4*>(&s_bias[c0 + c4]);
-#pragma unroll
-                for (int j = 0; j < 4; ++j) {
-                    const int r = j * 8 + r_in;
-                    if (r < rows_ok) {
-                        float4 x = *reinterpret_cast<const float4*>(scratch + r * kRbScratchLd + c4);
-                        x.x += bb.x; x.y += bb.y; x.z += bb.z; x.w += bb.w;
-                        *reinterpret_cast<float4*>(yb + (long)r * 128 + c0 + c4) = x;
-                    }
-                }
-                __syncwarp();
+                for (int j = 0; j < 16; ++j)
+                    if (r0 + j < rows_tile) yc[(long)(r0 + j) * 128] = v[j] + bias;
             }
         }
     }
     tc_fence_before();
     __syncthreads();
-    if (warp == 0) tmem_dealloc(tmem, tmem_cols);
+    if (warp == 0) tmem_dealloc(tmem, 256);
 }
 
 template <int KW, int TR>
 static int launch_rb_fwd(RbFwdParams& p, cudaStream_t st) {
-    const size_t smem = (size_t)4 * kRbTile + (size_t)kRbRawRows * 512 + (size_t)kRbEpi * 32 * kRbScratchLd * sizeof(float);
+    const size_t smem = (size_t)4 * kRbTile + (size_t)kRbRawRows * 512;
     static bool attr = false;
     if (!attr) {
         if (cudaFuncSetAttribute(resblock1d_fwd_kernel<KW, TR>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) {
@@ -358,20 +285,18 @@ static int launch_rb_fwd(RbFwdParams& p, cudaStream_t st) {
 // O recomputed from raw X for the 48 interior rows -> image, whose halo rows are zeroed once), 1 MMA warp, 8 epilogue warps.
 // Wpw^T is the TMEM-resident A operand of the data-gradient product (written once per CTA with tcgen05.st): the 64 KB its
 // shared-memory images would take hold a third raw X and a second raw dY buffer (the epilogue of tile i still reads X(i) while
-// tiles i + 1, i + 2 are prepared).  NPF_RB_BWD_TW = 0 keeps the weights in shared memory (two X buffers, one dY buffer).
+// tiles i + 1, i + 2 are prepared).
 // ------------------------------------------------------------------------------------------------------------------
 constexpr int kRwRows = 64;
 constexpr int kRwInt = 48;                                      // interior rows per tile (k = 11: 48 + 2 * 5 = 58 <= 64)
-// NE epilogue warps: 8 = two row groups of 24 interior rows (two 12-row sub-passes each), 12 = three row groups of 16 rows (one pass)
-constexpr int rw_threads(int NE) { return (kRbEpiWarp0 + NE + 1) * 32; }       // 832 / 960: producers + MMA + epilogue + loader warp
+constexpr int kRwThreads = (kRbEpiWarp0 + kRbEpi + 1) * 32;   // 832: producers + MMA + epilogue + loader warp
 constexpr uint32_t kRwHalf = 64u * 128u * 2u;                   // one bf16 64 x 128 image: 16 KB
+constexpr int kRwNX = 3, kRwNY = 2;                             // raw X / raw dY buffers in flight
 
 struct RbBwdParams {
     const float* dY; const float* X; const float* wdw; const float* bdw; const float* wpw;
     float* dX; float* dWdw; float* dbdw; float* dWpw; float* dbpw;
     int B, L, n_lt, n_tiles;
-    int tmem_w;          // 1: Wpw^T is the TMEM-resident A operand of the data-gradient product; the 64 KB its shared-memory images took
-                         //    hold a third raw X buffer and a second raw dY buffer instead
     unsigned long long* trace;
 };
 
@@ -397,13 +322,14 @@ __device__ __forceinline__ uint32_t rw_img_off(uint32_t m, uint32_t c) {
     return (c >> 6) * 8192u + m * 128u + ((((c & 63u) >> 3) ^ (m & 7u)) << 4) + (c & 7u) * 2u;
 }
 
+// NE = 8 epilogue warps: two row groups of 24 interior rows, two 12-row sub-passes each
 template <int KW, int NE>
-__global__ void __launch_bounds__(rw_threads(NE), 1) resblock1d_bwd_kernel(RbBwdParams p) {
+__global__ void __launch_bounds__(kRwThreads, 1) resblock1d_bwd_kernel(RbBwdParams p) {
     constexpr int P = KW / 2;
     constexpr int kRwLoadWarp = kRbEpiWarp0 + NE;
-    constexpr int NP = NE == 8 ? 2 : 1;                         // sub-passes per epilogue thread
-    constexpr int RP = NE == 8 ? 12 : 16;                       // interior rows per sub-pass
-    static_assert(NE == 8 || NE == 12, "epilogue warps: 8 or 12");
+    constexpr int NP = 2;                                       // sub-passes per epilogue thread
+    constexpr int RP = 12;                                      // interior rows per sub-pass
+    static_assert(NE == kRbEpi, "epilogue warps");
     static_assert((NE / 4) * NP * RP == kRwInt, "row groups must tile the interior");
     static_assert(kRwInt + 2 * P <= kRwRows, "tile too small for the halo");
     extern __shared__ __align__(1024) uint8_t smem_raw[];
@@ -411,19 +337,15 @@ __global__ void __launch_bounds__(rw_threads(NE), 1) resblock1d_bwd_kernel(RbBwd
     __shared__ uint32_t tmem_slot;
     __shared__ float s_db[128];
 
-    const bool TW = p.tmem_w != 0;
-    const int NX = TW ? 3 : 2, NY = TW ? 2 : 1;                 // raw X / raw dY buffers in flight
+    constexpr int NX = kRwNX, NY = kRwNY;
     constexpr int TILE = kRwRows * 128;                         // floats of one raw tile (32 KB)
     uint8_t* y_hi = smem_raw;                                   // dY image: hi 16 KB | lo 16 KB
     uint8_t* o_hi = smem_raw + 2 * kRwHalf;                     // O image
-    uint8_t* w_hi = smem_raw + 4 * kRwHalf;                     // Wpw: hi 32 KB | lo 32 KB   (only when Wpw is NOT kept in TMEM)
-    uint8_t* w_lo = w_hi + kRbTile;
-    float* rawY = reinterpret_cast<float*>(smem_raw + 4 * kRwHalf + (TW ? 0 : 2 * kRbTile));   // NY x [64][128]
-    float* rawX = rawY + NY * TILE;                                                             // NX x [64][128]
+    float* rawY = reinterpret_cast<float*>(smem_raw + 4 * kRwHalf);   // NY x [64][128]
+    float* rawX = rawY + NY * TILE;                                   // NX x [64][128]
 
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const uint32_t tmem_cols = TW ? 512u : 256u;
-    if (warp == 0) tmem_alloc(&tmem_slot, tmem_cols);
+    if (warp == 0) tmem_alloc(&tmem_slot, 512);
     if (tid == 32) {
         mbar_init(&bar_afull, kRbProd * 32);
         mbar_init(&bar_aempty, 1);
@@ -445,49 +367,34 @@ __global__ void __launch_bounds__(rw_threads(NE), 1) resblock1d_bwd_kernel(RbBwd
     const int per = p.n_tiles / (int)gridDim.x, rem = p.n_tiles - per * (int)gridDim.x;
     const int g0 = (int)blockIdx.x * per + min((int)blockIdx.x, rem), g1 = g0 + per + ((int)blockIdx.x < rem ? 1 : 0);
     pdl_trigger();
-    if (!TW && warp < kRbProd) {   // pointwise weights: warp w stages rows 8 w .. 8 w + 7 of Wpw[n][k] (two 64-column atoms of 16 KB)
-        const uint32_t pchunk = (uint32_t)(lane >> 1) & 7u;
-        const uint32_t woff = (uint32_t)(lane >> 4) * 16384u + (uint32_t)(warp * 8) * 128u + (uint32_t)(lane & 1) * 8u;
-#pragma unroll
-        for (int i = 0; i < 8; ++i) {
-            const float4 v = __ldg(reinterpret_cast<const float4*>(p.wpw + (long)(warp * 8 + i) * 128) + lane);
-            const uint32_t off = woff + (uint32_t)i * 128u + ((pchunk ^ (uint32_t)i) << 4);
-            const uint32_t h01 = pack_bf16(v.x, v.y), h23 = pack_bf16(v.z, v.w);
-            *reinterpret_cast<uint2*>(w_hi + off) = make_uint2(h01, h23);
-            *reinterpret_cast<uint2*>(w_lo + off) = make_uint2(pack_bf16(v.x - __uint_as_float(h01 << 16), v.y - __uint_as_float(h01 & 0xFFFF0000u)),
-                                                                 pack_bf16(v.z - __uint_as_float(h23 << 16), v.w - __uint_as_float(h23 & 0xFFFF0000u)));
-        }
-    }
     fence_async_smem();
     tc_fence_before();
     __syncthreads();
     tc_fence_after();
     const uint32_t tmem = tmem_slot;
-    if (TW) {
-        // Wpw^T as the TMEM-resident A operand of dO^T = Wpw^T . dY^T: lane k = input channel k holds column k of Wpw [n, k] (K-major over
-        // the output channel n, two consecutive n per 32-bit column), hi at columns [256, 320), lo at [320, 384)
-        if (warp < 4) {
-            const float* wc = p.wpw + 32 * warp + lane;
-            const uint32_t tw = tmem + ((uint32_t)(32 * warp) << 16) + 256u;
+    // Wpw^T as the TMEM-resident A operand of dO^T = Wpw^T . dY^T: lane k = input channel k holds column k of Wpw [n, k] (K-major over
+    // the output channel n, two consecutive n per 32-bit column), hi at columns [256, 320), lo at [320, 384)
+    if (warp < 4) {
+        const float* wc = p.wpw + 32 * warp + lane;
+        const uint32_t tw = tmem + ((uint32_t)(32 * warp) << 16) + 256u;
 #pragma unroll 1
-            for (int cc = 0; cc < 4; ++cc) {
-                uint32_t hi[16], lo[16];
+        for (int cc = 0; cc < 4; ++cc) {
+            uint32_t hi[16], lo[16];
 #pragma unroll
-                for (int i = 0; i < 16; ++i) {
-                    const float v0 = __ldg(wc + (long)(32 * cc + 2 * i) * 128), v1 = __ldg(wc + (long)(32 * cc + 2 * i + 1) * 128);
-                    const uint32_t h = pack_bf16(v0, v1);
-                    hi[i] = h;
-                    lo[i] = pack_bf16(v0 - __uint_as_float(h << 16), v1 - __uint_as_float(h & 0xFFFF0000u));
-                }
-                tmem_st16(tw + (uint32_t)(cc * 16), hi);
-                tmem_st16(tw + 64u + (uint32_t)(cc * 16), lo);
+            for (int i = 0; i < 16; ++i) {
+                const float v0 = __ldg(wc + (long)(32 * cc + 2 * i) * 128), v1 = __ldg(wc + (long)(32 * cc + 2 * i + 1) * 128);
+                const uint32_t h = pack_bf16(v0, v1);
+                hi[i] = h;
+                lo[i] = pack_bf16(v0 - __uint_as_float(h << 16), v1 - __uint_as_float(h & 0xFFFF0000u));
             }
-            tmem_st_wait();
+            tmem_st16(tw + (uint32_t)(cc * 16), hi);
+            tmem_st16(tw + 64u + (uint32_t)(cc * 16), lo);
         }
-        tc_fence_before();
-        __syncthreads();
-        tc_fence_after();
+        tmem_st_wait();
     }
+    tc_fence_before();
+    __syncthreads();
+    tc_fence_after();
     pdl_wait();
 
     if (warp == kRwLoadWarp) {
@@ -612,13 +519,10 @@ __global__ void __launch_bounds__(rw_threads(NE), 1) resblock1d_bwd_kernel(RbBwd
     } else if (warp == kRbMmaWarp) {
         // ------------------------------------------------------------------ MMA issuer
         if (lane == 0) {
-            const uint32_t idesc_dx = make_idesc(128, 64, 1, 0);      // A = Wpw^T (MN-major view), B = dY tile (K-major), D = dO^T [k x m]
-            const uint32_t idesc_dx_ts = make_idesc(128, 64, 0, 0);   // the same product with A = Wpw^T stored K-major in TMEM
+            const uint32_t idesc_dx_ts = make_idesc(128, 64, 0, 0);   // A = Wpw^T stored K-major in TMEM, B = dY tile (K-major), D = dO^T [k x m]
             const uint32_t idesc_dw = make_idesc(128, 128, 1, 1);     // A = dY^T, B = O: MN-major views (reduction over the tile's rows)
-            const uint32_t sw_hi = smem_u32(w_hi), sw_lo = smem_u32(w_lo);
             const uint32_t sy_hi = smem_u32(y_hi), sy_lo = sy_hi + kRwHalf, so_hi = smem_u32(o_hi), so_lo = so_hi + kRwHalf;
-            // base descriptors, built once: W^T (MN-major view), dY K-major (data gradient), dY^T / O MN-major (weight gradient)
-            const uint64_t dw_h = rb_desc_sw128(sw_hi, 16384, 1024), dw_l = rb_desc_sw128(sw_lo, 16384, 1024);
+            // base descriptors, built once: dY K-major (data gradient), dY^T / O MN-major (weight gradient)
             const uint64_t dyk_h = rb_desc_sw128(sy_hi, 16, 1024), dyk_l = rb_desc_sw128(sy_lo, 16, 1024);
             const uint64_t dym_h = rb_desc_sw128(sy_hi, 8192, 1024), dym_l = rb_desc_sw128(sy_lo, 8192, 1024);
             const uint64_t dom_h = rb_desc_sw128(so_hi, 8192, 1024), dom_l = rb_desc_sw128(so_lo, 8192, 1024);
@@ -637,17 +541,10 @@ __global__ void __launch_bounds__(rw_threads(NE), 1) resblock1d_bwd_kernel(RbBwd
                 for (int ks = 0; ks < 8; ++ks) {
                     const uint32_t bo = (uint32_t)(ks >> 2) * 8192u + (uint32_t)(ks & 3) * 32u;
                     const uint64_t b_h = desc_adv(dyk_h, bo);
-                    if (TW) {            // A = Wpw^T from TMEM (8 columns per 16-wide slice of the reduction over n)
-                        const uint32_t ta = tmem + 256u + (uint32_t)ks * 8u;
-                        umma_bf16_ts(d_dx, ta, b_h, idesc_dx_ts, ks ? 1u : 0u);
-                        umma_bf16_ts(d_dx, ta, desc_adv(dyk_l, bo), idesc_dx_ts, 1);
-                        umma_bf16_ts(d_dx, ta + 64u, b_h, idesc_dx_ts, 1);
-                    } else {
-                        const uint64_t a_h = desc_adv(dw_h, ks * 2048u);
-                        umma_bf16(d_dx, a_h, b_h, idesc_dx, ks ? 1u : 0u);
-                        umma_bf16(d_dx, a_h, desc_adv(dyk_l, bo), idesc_dx, 1);
-                        umma_bf16(d_dx, desc_adv(dw_l, ks * 2048u), b_h, idesc_dx, 1);
-                    }
+                    const uint32_t ta = tmem + 256u + (uint32_t)ks * 8u;    // A = Wpw^T from TMEM (8 columns per 16-wide slice of the reduction over n)
+                    umma_bf16_ts(d_dx, ta, b_h, idesc_dx_ts, ks ? 1u : 0u);
+                    umma_bf16_ts(d_dx, ta, desc_adv(dyk_l, bo), idesc_dx_ts, 1);
+                    umma_bf16_ts(d_dx, ta + 64u, b_h, idesc_dx_ts, 1);
                 }
                 umma_commit(&bar_tfull[a]);
 #pragma unroll
@@ -686,8 +583,8 @@ __global__ void __launch_bounds__(rw_threads(NE), 1) resblock1d_bwd_kernel(RbBwd
             if (e == 0 && lane == 0) trace_ev(p.trace, 2, 2);
 #pragma unroll
             for (int sp = 0; sp < NP; ++sp) {                    // sub-passes of RP interior rows: dO window of RP + 2 P rows
-                const int c = (NP * RP) * h + RP * sp;           // first tile row (= accumulator column) of the window: 0, 12, 24, 36 / 0, 16, 32
-                const int OFF = NE == 8 ? 4 * sp : 0;            // the window starts at d[OFF]: ...
+                const int c = (NP * RP) * h + RP * sp;           // first tile row (= accumulator column) of the window: 0, 12, 24, 36
+                const int OFF = 4 * sp;                          // the window starts at d[OFF]: ...
                 const int cs = c - OFF;                           // ... it is fetched from the 8-aligned column at or below it
                 float d[32];
                 {
@@ -735,10 +632,9 @@ __global__ void __launch_bounds__(rw_threads(NE), 1) resblock1d_bwd_kernel(RbBwd
         // ---- flush of the CTA's pointwise weight gradient: thread = row n of dWpw, 64 columns per warp
         mbar_wait(&bar_dwfull, 0);
         tc_fence_after();
-        const int col_base = NE == 8 ? h * 64 : h * 48;           // 128 columns over the row groups: 64 + 64 or 48 + 48 + 32
-        const int n_ch = NE == 8 ? 4 : (h < 2 ? 3 : 2);
+        const int col_base = h * 64;                              // 128 columns over the two row groups
 #pragma unroll 1
-        for (int ch = 0; ch < n_ch; ++ch) {
+        for (int ch = 0; ch < 4; ++ch) {
             const int c0 = col_base + ch * 16;
             float v[16];
             tmem_ld16(tmem + ((uint32_t)lane_base << 16) + (uint32_t)(128 + c0), v);
@@ -749,12 +645,12 @@ __global__ void __launch_bounds__(rw_threads(NE), 1) resblock1d_bwd_kernel(RbBwd
     }
     tc_fence_before();
     __syncthreads();
-    if (warp == 0) tmem_dealloc(tmem, tmem_cols);
+    if (warp == 0) tmem_dealloc(tmem, 512);
 }
 
 template <int KW, int NE>
 static int launch_rb_bwd(RbBwdParams& p, cudaStream_t st) {
-    const size_t smem = (size_t)4 * kRwHalf + 2 * kRbTile + (size_t)3 * kRwRows * 512;
+    const size_t smem = (size_t)4 * kRwHalf + (size_t)(kRwNY + kRwNX) * kRwRows * 512;
     static bool attr = false;
     if (!attr) {
         if (cudaFuncSetAttribute(resblock1d_bwd_kernel<KW, NE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) {
@@ -764,7 +660,7 @@ static int launch_rb_bwd(RbBwdParams& p, cudaStream_t st) {
         attr = true;
     }
     const int grid = p.n_tiles < kNumSMs ? p.n_tiles : kNumSMs;
-    launch_pdl(resblock1d_bwd_kernel<KW, NE>, dim3(grid), dim3(rw_threads(NE)), smem, st, p);
+    launch_pdl(resblock1d_bwd_kernel<KW, NE>, dim3(grid), dim3(kRwThreads), smem, st, p);
     count_launch();
     return check_launch("resblock1d_bwd_kernel");
 }
@@ -780,24 +676,17 @@ extern "C" int npf_resblock1d_fwd(const float* X, const float* wdw, const float*
     NPF_REQUIRE(X && wdw && wpw && Y, "npf_resblock1d_fwd: null pointer");
     NPF_REQUIRE(B >= 0 && L >= 1 && k >= 1 && (k & 1), "npf_resblock1d_fwd: bad shape (odd kernel size)");
     if (B == 0) return NPF_OK;
-    static const bool on = [] { const char* e = getenv("NPF_RESBLOCK_FUSED"); return !(e && e[0] == '0'); }();
-    if (!on || C != 128 || precision != NPF_PREC_BF16X3 || k != 11 || !rb_aligned16(X) || !rb_aligned16(Y) || !rb_aligned16(wpw) || (O && !rb_aligned16(O))) {
+    if (C != 128 || precision != NPF_PREC_BF16X3 || k != 11 || !rb_aligned16(X) || !rb_aligned16(Y) || !rb_aligned16(wpw) || (O && !rb_aligned16(O))) {
         set_error("npf_resblock1d_fwd: covered: 128 channels, kernel size 11, precision bf16x3, 16-byte aligned tensors; run npf_dwconv_fwd + npf_linear_fwd otherwise");
         return NPF_ENOTSUP;
     }
     RbFwdParams p{};
     p.X = X; p.wdw = wdw; p.bdw = bdw; p.wpw = wpw; p.bpw = bpw; p.O = O; p.Y = Y; p.B = B; p.L = L;
-    // rows per tile: the choice that leaves the fewest rows on the most loaded CTA (96 needs the transposed product: rows = N extent)
-    static const int tr_env = [] { const char* e = getenv("NPF_RB_FWD_TR"); return e ? atoi(e) : 0; }();
+    // rows per tile: the choice that leaves the fewest rows on the most loaded CTA
     auto critical_rows = [&](int tr) { const long nt = (long)B * ((L + tr - 1) / tr); return ((nt + kNumSMs - 1) / kNumSMs) * tr; };
-    int tr = 128;
-    if (tr_env == 96 || (tr_env == 0 && critical_rows(96) < critical_rows(128))) tr = 96;
+    const int tr = critical_rows(96) < critical_rows(128) ? 96 : 128;
     p.n_lt = (L + tr - 1) / tr;
     p.n_tiles = B * p.n_lt;
-    // product orientation: 1 (default) = Y^T = Wpw . O^T, rows stored straight from the TMEM registers (39.5 us per launch at config 2);
-    // 0 = Y = O . Wpw^T with a shared-memory transpose in the epilogue (45.3 us); 2 = as 1 with Wpw read from TMEM (42.8 us)
-    static const int tr_mode = [] { const char* e = getenv("NPF_RB_FWD_T"); const int v = e ? atoi(e) : 1; return v >= 0 && v <= 2 ? v : 1; }();
-    p.transposed = tr == 96 && tr_mode == 0 ? 1 : tr_mode;
     p.trace = trace_buffer();
     return tr == 96 ? launch_rb_fwd<11, 96>(p, as_stream(stream)) : launch_rb_fwd<11, 128>(p, as_stream(stream));
 }
@@ -807,8 +696,7 @@ extern "C" int npf_resblock1d_bwd(const float* dY, const float* X, const float* 
     NPF_REQUIRE(dY && X && wdw && wpw && dX && dWdw && dWpw, "npf_resblock1d_bwd: null pointer");
     NPF_REQUIRE(B >= 0 && L >= 1 && k >= 1 && (k & 1), "npf_resblock1d_bwd: bad shape (odd kernel size)");
     if (B == 0) return NPF_OK;
-    static const bool on = [] { const char* e = getenv("NPF_RESBLOCK_FUSED"); return !(e && e[0] == '0'); }();
-    if (!on || C != 128 || precision != NPF_PREC_BF16X3 || k != 11 || !rb_aligned16(dY) || !rb_aligned16(X) || !rb_aligned16(dX) || !rb_aligned16(wpw) ||
+    if (C != 128 || precision != NPF_PREC_BF16X3 || k != 11 || !rb_aligned16(dY) || !rb_aligned16(X) || !rb_aligned16(dX) || !rb_aligned16(wpw) ||
         !rb_aligned16(dWpw)) {
         set_error("npf_resblock1d_bwd: covered: 128 channels, kernel size 11, precision bf16x3, 16-byte aligned tensors; run npf_linear_bwd + npf_dwconv_bwd otherwise");
         return NPF_ENOTSUP;
@@ -818,9 +706,6 @@ extern "C" int npf_resblock1d_bwd(const float* dY, const float* X, const float* 
     p.B = B; p.L = L;
     p.n_lt = (L + kRwInt - 1) / kRwInt;
     p.n_tiles = B * p.n_lt;
-    static const int tw = [] { const char* e = getenv("NPF_RB_BWD_TW"); return e ? (e[0] != '0' ? 1 : 0) : 1; }();
-    p.tmem_w = tw;
     p.trace = trace_buffer();
-    static const int ne = [] { const char* e = getenv("NPF_RB_BWD_EPI"); return e && atoi(e) == 12 ? 12 : 8; }();
-    return ne == 12 ? launch_rb_bwd<11, 12>(p, as_stream(stream)) : launch_rb_bwd<11, 8>(p, as_stream(stream));
+    return launch_rb_bwd<11, kRbEpi>(p, as_stream(stream));
 }

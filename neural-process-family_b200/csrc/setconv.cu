@@ -10,7 +10,6 @@
 //
 // Generic kernels (any K, Q, C <= 256).  The shared-memory/TMA-staged fast path for the induced->target direction
 // is in setconv_tile.cu.
-#include <cstdlib>
 #include "common.cuh"
 
 namespace npf {
@@ -485,10 +484,7 @@ __global__ void __launch_bounds__(256) setconv_sorted_kernel(const float* __rest
     }
 }
 
-static bool sorted_ok(int K) {
-    static const bool on = [] { const char* e = getenv("NPF_SETCONV_SORTED"); return !(e && e[0] == '0'); }();
-    return on && K <= kSortedMaxK;
-}
+static bool sorted_ok(int K) { return K <= kSortedMaxK; }
 
 // implemented in setconv_tile.cu: shared-memory staged fast path; NPF_ENOTSUP if the shape is not covered
 int setconv_tile_fwd(const float* keys, long key_bs, const float* queries, long qry_bs, const float* values,

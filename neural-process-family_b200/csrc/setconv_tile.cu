@@ -11,7 +11,6 @@
 //   mode 0: feat = sum_k softmax_k(a) V_k, dens, (max logit, sum exp)            (forward)
 //   mode 1: d theta: T - G*A1 + ddens*A2 with max-shifted logits (see setconv.cu)
 //   dV    : dV[k] = sum_q w_qk dF_q                                               (gather, no atomics)
-#include <cstdlib>
 #include "tc_common.cuh"
 
 namespace npf {
@@ -1248,14 +1247,12 @@ __global__ void __launch_bounds__(kBwThreads, 1) setconv_tc_bwd_kernel(const flo
 }
 
 static bool tc_bwd_ok(int K, int Q, int C, long key_bs) {
-    static const bool on = [] { const char* e = getenv("NPF_SETCONV_TC_BWD"); return !(e && e[0] == '0'); }();
-    return on && C == 128 && key_bs == 0 && K >= 3 && K <= kMaxChunks * kChunkRows && Q >= 1 && Q <= 128;
+    return C == 128 && key_bs == 0 && K >= 3 && K <= kMaxChunks * kChunkRows && Q >= 1 && Q <= 128;
 }
 
 static bool tc_fwd_ok(int K, int Q, int C, long key_bs) {
-    static const bool on = [] { const char* e = getenv("NPF_SETCONV_TC"); return !(e && e[0] == '0'); }();
     (void)Q;
-    return on && C == 128 && key_bs == 0 && K <= kMaxChunks * kChunkRows && K > 2 * kTcKeys;     // >= 3 chunks: the per-unit denominators are double-buffered against the 2-stage ring
+    return C == 128 && key_bs == 0 && K <= kMaxChunks * kChunkRows && K > 2 * kTcKeys;     // >= 3 chunks: the per-unit denominators are double-buffered against the 2-stage ring
 }
 
 static size_t task_smem_fwd(int K, int Q) {

@@ -9,10 +9,11 @@ one host call per step, kernels back to back on the device.
     loss = step(X_cntxt, Y_cntxt, X_trgt, Y_trgt)   # gradients are in p.grad (views of step.flat.flat) afterwards
     optimizer.step()
 
-What is captured: ``flat.zero_()``, ``model(...)``, ``criterion(...)``, ``loss.backward()`` (and, with
-``NPF_GRAPH_ALLREDUCE=1``, the flat-gradient all-reduce).  What stays outside: the host->device copies of the inputs into the
-graph's static buffers, the flat-gradient all-reduce (default; NCCL ``ReduceOp.AVG`` right after the replay), the optimizer, and the host side of the asynchronous [-1, 1] range validation (``_validate_inputs`` only launches the check
-kernel while capturing; the flag is read back after every replay).
+What is captured: ``flat.zero_()``, ``model(...)``, ``criterion(...)``, ``loss.backward()`` (and, when the one-kernel NVLink
+all-reduce ``parallel.P2PAllReduce`` is set up, the flat-gradient all-reduce).  What stays outside: the host->device copies of
+the inputs into the graph's static buffers, the NCCL flat-gradient all-reduce otherwise (``ReduceOp.AVG`` right after the
+replay), the optimizer, and the host side of the asynchronous [-1, 1] range validation (``_validate_inputs`` only launches the
+check kernel while capturing; the flag is read back after every replay).
 
 Constraints (the usual ones of whole-network capture): shapes are static per graph -- a new (n_cntxt, n_trgt, batch)
 signature records a new graph (LRU cache of ``max_graphs``); Python-side control flow is frozen at capture (number of
@@ -41,13 +42,10 @@ class GraphedStep:
                                       "thread inside backward; run that configuration eagerly")
         self.flat = flat if flat is not None else FlatGradients(model)
         self.n_warmup, self.max_graphs = n_warmup, max_graphs
-        import os
-        # where the gradient all-reduce of a multi-GPU step runs: inside the recorded graph, or right after the replay on the
-        # caller's stream (NPF_GRAPH_ALLREDUCE=0/1; measured at N=2 on B200, profiles/r2/allreduce_placement.md)
-        # Default: the one-kernel NVLink all-reduce (parallel.P2PAllReduce) is recorded into the graph (0.758 vs 0.762 ms at N=2); the NCCL
-        # fallback runs after the replay (no difference measured either way).
-        dflt = "1" if getattr(self.flat, "p2p", None) is not None else "0"
-        self.allreduce_in_graph = os.environ.get("NPF_GRAPH_ALLREDUCE", dflt) == "1"
+        # where the gradient all-reduce of a multi-GPU step runs: the one-kernel NVLink all-reduce (parallel.P2PAllReduce) is
+        # recorded into the graph (0.758 vs 0.762 ms at N=2 on B200, profiles/r2/allreduce_placement.md); the NCCL fallback runs
+        # right after the replay on the caller's stream (no difference measured either way)
+        self.allreduce_in_graph = getattr(self.flat, "p2p", None) is not None
         self._graphs = OrderedDict()
         self._side = None
 

@@ -59,10 +59,9 @@ class P2PAllReduce:
         self._in = (ctypes.c_void_p * self.world)(*ins)
         self._sig = (ctypes.c_void_p * self.world)(*sigs)
         self._out = (ctypes.c_void_p * self.world)(*outs)
-        import os
         # two-shot (each rank reduces one slice and writes it to everybody) from 4 ranks up, one-shot (everybody reads everything) below:
         # measured on B200 NVLink, profiles/r2/allreduce_placement.md
-        self.two_shot = os.environ.get("NPF_P2P_TWO_SHOT", "1" if self.world >= 4 else "0") == "1"
+        self.two_shot = self.world >= 4
         self.bucket = torch.as_tensor(_DevMem(mine[0], n, "<f4"), device=device)
         self.out = torch.as_tensor(_DevMem(mine[1], n, "<f4"), device=device)
         dist.barrier(group=group)                                          # every rank has opened every handle before the first launch
@@ -96,8 +95,7 @@ class P2PAllReduce:
 
 def _try_p2p(numel, device, group):
     """P2PAllReduce if every rank of the group can set it up (same node, peer access), else None -- decided collectively."""
-    import os
-    if os.environ.get("NPF_P2P_ALLREDUCE", "1") == "0" or device.type != "cuda" or dist.get_backend(group) != "nccl":
+    if device.type != "cuda" or dist.get_backend(group) != "nccl":
         return None
     p2p, ok = None, 1
     try:
@@ -169,8 +167,7 @@ class FlatGradients:
         if self.p2p is not None:
             self.p2p.reduce_()
             return self.flat
-        import os
-        if self.flat.is_cuda and os.environ.get("NPF_ALLREDUCE_AVG", "1") == "1":      # NCCL averages inside the collective: no separate 1/G kernel
+        if self.flat.is_cuda:      # NCCL averages inside the collective: no separate 1/G kernel
             dist.all_reduce(self.flat, op=dist.ReduceOp.AVG, group=self.group)
         else:                      # gloo (CPU host-logic tests) has no AVG
             dist.all_reduce(self.flat, op=dist.ReduceOp.SUM, group=self.group)

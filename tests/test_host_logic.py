@@ -110,6 +110,17 @@ def test_product_does_not_import_oracle():
                 assert "oracle" not in src.replace("no oracle", ""), f"{f} references the oracle"
 
 
+def test_product_does_not_read_environment():
+    # every kernel choice follows from what the code observes (shapes, precision, alignment, capture, world size): a variable
+    # that selects a path nobody tests would let an untested kernel run
+    pkg = os.path.join(ROOT, "neural-process-family_b200")
+    for dirpath, _, files in os.walk(pkg):
+        for f in files:
+            if f.endswith((".cu", ".cuh", ".py")):
+                src = open(os.path.join(dirpath, f)).read()
+                assert "getenv" not in src and "environ" not in src, f"{f} reads the environment"
+
+
 def test_sync_batchnorm_marks_modules_and_graphed_step_refuses():
     import torch.nn as nn
     from functools import partial
