@@ -4,6 +4,7 @@ import glob
 import os
 import sys
 
+import pytest
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -164,3 +165,9 @@ def rel_err(a, b):
     if a.numel() == 0:
         return 0.0
     return ((a - b).abs().max() / b.abs().max().clamp_min(1e-30)).item()
+
+
+def keep_ids(cases, default):
+    """pytest.params whose id leaves out the last column when it holds `default`: the cases that existed before that
+    column was added keep their test ids."""
+    return [pytest.param(*c, id="-".join(map(str, c if c[-1] != default else c[:-1]))) for c in cases]

@@ -1,14 +1,27 @@
 """-m gpu: the tcgen05 / TMEM tensor-core path of the linear layers (NPF_PREC_BF16, NPF_PREC_BF16X3) against fp64
-torch: the 3-term split-bf16 mode must meet the fp32 bar (1e-4), plain bf16 the 1e-2 bar of the north star."""
+torch: the 3-term split-bf16 mode must meet the fp32 bar (1e-4), plain bf16 the 1e-2 bar of the north star.
+
+Gradient bars.  Where every ReLU mask comes from an input the test supplies (so fp32 and fp64 agree on it), the gradient
+error is the arithmetic alone and the bar is set from the worst error measured on a B200, about 4x that rounded up:
+GBARS (L2) and GMAX (max-rel).  Split-bf16 with all three products errs by ~5e-6 there, with one correction product
+lost by ~2e-3 (CPU emulation, tests/test_tc_bars.py), so these bars tell the two apart.  test_tc_mlp_chain computes its
+masks from fp32 pre-activations and keeps the looser ReLU-flip bar of BARS."""
 import pytest
 import torch
 import torch.nn.functional as F
 
 from _cfg import build_model, loss_for
-from _util import load_fixture, rel_err
+from _util import keep_ids, load_fixture, rel_err
 
 pytestmark = pytest.mark.gpu
-BARS = {"bf16": (1e-2, 2e-1), "bf16x3": (1e-4, 3e-3)}   # (forward max-rel, gradient L2-rel) tolerances
+BARS = {"bf16": (1e-2, 2e-1), "bf16x3": (1e-4, 3e-3)}   # (forward max-rel, gradient L2-rel with ReLU flips) tolerances
+# flip-free gradient bars; worst error measured on a B200 (bf16x3 / bf16) in the comment.  The one-layer bar is 5e-5
+# rather than 2e-5 so that it stays 5x above the emulated split-bf16 error (4.5e-6; tests/test_tc_bars.py)
+GBARS = {"bf16x3": 5e-5, "bf16": 1e-2}          # L2-rel, one layer (npf_linear_bwd): 4.7e-6 / 2.4e-3
+CHAIN_GBARS = {"bf16x3": 1e-4, "bf16": 5e-2}    # L2-rel, npf_mlp_chain_bwd (up to 8 layers): 1.3e-5 / 6.7e-3
+GMAX = {"bf16x3": 5e-5}                         # max-rel, one layer through npf_b200.ops.linear: 7.9e-6
+ABARS = {"bf16x3": 5e-5, "bf16": 2e-2}          # L2-rel, attention: 7.2e-6 / 4.9e-3
+ZERO_GRAD_BARS = {"bf16x3": 2e-3, "bf16": 5e-2}  # attention gradients that are 0 analytically: cancellation only, 3.3e-4 / 2.7e-2
 
 
 def l2_rel(a, b):
@@ -17,6 +30,11 @@ def l2_rel(a, b):
     units happen to sit within 1e-5 of zero, not the arithmetic."""
     a, b = a.detach().double().cpu(), b.detach().double().cpu()
     return ((a - b).norm() / b.norm().clamp_min(1e-30)).item()
+
+
+def grad_max_rel(a, b):
+    """max |a - b| / max |b| of a gradient (rel_err under its own name, so each bar's metric reads at the call)."""
+    return rel_err(a, b)
 
 
 @pytest.fixture(scope="module")
@@ -61,7 +79,7 @@ def test_tc_fused_linear_backward(npf, prec, M, mask, bias):
     from npf_b200 import _cabi
     K = N = 128
     pr = {"bf16": 1, "bf16x3": 2}[prec]
-    _, gtol = BARS[prec]
+    gtol = GBARS[prec]
     dY, W = _g(M, N, seed=1), _g(N, K, seed=2, scale=K ** -0.5)
     X = torch.relu(_g(M, K, seed=3))
     dW0, db0 = _g(N, K, seed=4), _g(N, seed=5)
@@ -138,7 +156,7 @@ def test_tc_mlp_chain_bwd_entry(npf, prec, L, M, need_dx, mask0):
     import ctypes
     from npf_b200 import _cabi
     pr = {"bf16": 1, "bf16x3": 2}[prec]
-    _, gtol = BARS[prec]
+    gtol = CHAIN_GBARS[prec]
     st = torch.cuda.current_stream().cuda_stream
     Ws = [_g(128, 128, seed=10 + l, scale=128 ** -0.5) for l in range(L)]
     X0 = _g(M, 128, seed=1)
@@ -168,17 +186,17 @@ def test_tc_mlp_chain_bwd_entry(npf, prec, L, M, need_dx, mask0):
     torch.cuda.synchronize()
     if need_dx:
         assert torch.isfinite(dXc).all()
-        assert l2_rel(dXc, dz) < gtol * L, ("dX", l2_rel(dXc, dz))
+        assert l2_rel(dXc, dz) < gtol, ("dX", l2_rel(dXc, dz))
         if mask0:
             assert (dXc[Xc[0] <= 0] == 0).all()
     for l in range(L):
         e = l2_rel(dWc[l] - c(dW0[l]), dWr[l])
-        assert e < gtol * (L - l), (f"dW{l}", e)
+        assert e < gtol, (f"dW{l}", e)
         if l == skip_db:
             assert torch.equal(dbc[l], c(db0[l]))
         else:
             e = l2_rel(dbc[l] - c(db0[l]), dbr[l])
-            assert e < gtol * (L - l), (f"db{l}", e)
+            assert e < gtol, (f"db{l}", e)
 
 
 @pytest.mark.parametrize("prec", ["bf16x3", "bf16"])
@@ -207,7 +225,7 @@ def test_tc_single_linear_localised(npf, prec, M, K, N):
     """One layer at a time (forward, data gradient, weight gradient reported separately) + run-to-run determinism of
     the forward and of the data gradient (no atomics on those paths)."""
     npf.set_precision(prec)
-    ftol, gtol = BARS[prec]
+    ftol, gtol = BARS[prec][0], GMAX[prec]
     x, W, b = _g(M, K, seed=1), _g(N, K, seed=2, scale=K ** -0.5), _g(N, seed=3)
     go = _g(M, N, seed=4)
     res = []
@@ -217,39 +235,57 @@ def test_tc_single_linear_localised(npf, prec, M, K, N):
         yc.backward(go.float().cuda())
         res.append((yc.detach().clone(), xc.grad.clone(), Wc.grad.clone(), bc.grad.clone()))
     yr = x @ W.t() + b
-    errs = dict(y=rel_err(res[0][0], yr), dx=rel_err(res[0][1], go @ W), dW=rel_err(res[0][2], go.t() @ x), db=rel_err(res[0][3], go.sum(0)))
+    errs = dict(y=rel_err(res[0][0], yr), dx=grad_max_rel(res[0][1], go @ W), dW=grad_max_rel(res[0][2], go.t() @ x),
+                db=grad_max_rel(res[0][3], go.sum(0)))
     assert torch.equal(res[0][0], res[1][0]) and torch.equal(res[0][1], res[1][1]), f"non-deterministic: {errs}"
     assert errs["y"] < ftol and errs["dx"] < gtol and errs["dW"] < gtol and errs["db"] < gtol, errs
 
 
-@pytest.mark.parametrize("prec", ["bf16x3", "bf16"])
-@pytest.mark.parametrize("B,Tq,Tk,H,D", [(2, 128, 128, 8, 16), (1, 33, 70, 8, 16), (2, 300, 513, 4, 32), (1, 1, 1, 8, 16), (2, 512, 512, 8, 16)])
-def test_tc_attention_forward(npf, prec, B, Tq, Tk, H, D):
-    """tcgen05 attention forward + backward (head dim 16 / 32) vs fp64 softmax attention."""
+def attn_grad_err(a, b, gmax, floor):
+    """L2 error of one attention gradient relative to its own norm, floored at a fraction of the largest of the three
+    (with a single key the softmax gradient w.r.t. q and k is exactly 0: only cancellation is left to compare)."""
+    return (a.detach().double().cpu() - b).norm().item() / max(b.norm().item(), floor * gmax)
+
+
+def attn_ref(q, k, v, H, D, Dv):
+    """fp64 softmax attention over H heads; q, k [B, T, H*D], v [B, Tk, H*Dv]."""
     import math
+    heads = lambda t, d: t.view(t.shape[0], t.shape[1], H, d).transpose(1, 2)
+    s = heads(q, D) @ heads(k, D).transpose(-1, -2) / math.sqrt(D)
+    return (s.softmax(-1) @ heads(v, Dv)).transpose(1, 2).reshape(q.shape[0], q.shape[1], H * Dv)
+
+
+@pytest.mark.parametrize("prec", ["bf16x3", "bf16"])
+@pytest.mark.parametrize("B,Tq,Tk,H,D,Dv", keep_ids([
+    (2, 128, 128, 8, 16, None), (1, 33, 70, 8, 16, None), (2, 300, 513, 4, 32, None), (1, 1, 1, 8, 16, None), (2, 512, 512, 8, 16, None),
+    (38, 128, 100, 8, 16, None),    # 304 CTAs: 64-key chunks, a 36-key tail
+    (40, 130, 513, 8, 32, None),    # 64-key chunks with head dim 32, query and key tails
+    (2, 33, 70, 8, 16, 32), (1, 130, 150, 8, 32, 16),        # value head dim Dv != query / key head dim D, 128-key chunks
+    (40, 130, 100, 4, 16, 32), (40, 130, 100, 4, 32, 16),    # ... and with 64-key chunks (320 CTAs)
+], None))   # Dv None: the value head dim is D
+def test_tc_attention_forward(npf, prec, B, Tq, Tk, H, D, Dv):
+    """tcgen05 attention forward + backward (head dims 16 / 32, also mixed between q/k and v) vs fp64 softmax attention."""
+    import math
+    Dv = Dv or D
     npf.set_precision(prec)
     ftol = {"bf16x3": 1e-4, "bf16": 1e-2}[prec]
-    q, k, v = _g(B, Tq, H * D, seed=1), _g(B, Tk, H * D, seed=2), _g(B, Tk, H * D, seed=3)
-
-    def heads(t):
-        return t.view(t.shape[0], t.shape[1], H, D).transpose(1, 2)
-
+    q, k, v = _g(B, Tq, H * D, seed=1), _g(B, Tk, H * D, seed=2), _g(B, Tk, H * Dv, seed=3)
     r = [t.clone().requires_grad_(True) for t in (q, k, v)]
-    s = heads(r[0]) @ heads(r[1]).transpose(-1, -2) / math.sqrt(D)
-    yr = (s.softmax(-1) @ heads(r[2])).transpose(1, 2).reshape(B, Tq, H * D)
+    yr = attn_ref(*r, H, D, Dv)
     c = [t.float().cuda().requires_grad_(True) for t in (q, k, v)]
     yc = npf.ops.xattn(c[0], c[1], c[2], H, 1.0 / math.sqrt(D))
+    assert yc.shape == yr.shape
     assert rel_err(yc, yr) < ftol, (prec, rel_err(yc, yr))
     go = _g(*yr.shape, seed=9)
     yr.backward(go)
     yc.backward(go.float().cuda())
-    gtol = {"bf16x3": 2e-3, "bf16": 5e-2}[prec]
     gmax = max(t_.grad.norm().item() for t_ in r)
+    floor = {"bf16x3": 1e-2, "bf16": 5e-2}[prec]
     for n, a, b_ in zip("qkv", c, r):
-        # L2 error relative to the gradient's own norm, floored at a fraction of the largest of the three (with a single key the
-        # softmax gradient w.r.t. q and k is exactly 0)
-        err = (a.grad.double().cpu() - b_.grad).norm().item() / max(b_.grad.norm().item(), {"bf16x3": 1e-2, "bf16": 5e-2}[prec] * gmax)
-        assert err < gtol, f"{prec} grad {n}: {err}"
+        err = attn_grad_err(a.grad, b_.grad, gmax, floor)
+        # a gradient below the floor is 0 analytically (one key: dq = dk = 0) and what is left is cancellation
+        bar = ABARS[prec] if b_.grad.norm().item() >= floor * gmax else ZERO_GRAD_BARS[prec]
+        assert err < bar, f"{prec} grad {n}: {err}"
 
 
 from _util import fixture_names  # noqa: E402
